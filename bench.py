@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the hot path: 1080p CQP I+P H.264 encode, frames/s (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: the whole synthetic clip of the workload
 (default: BASELINE.json configs[2], 1920x1088 NV12, 600 frames, GOP 60, QP 25, +-16 full search,
@@ -15,6 +15,9 @@ raw frames and D2H of the bytestream inside the timed region.
 --impl reference times the CPU implementation of the same path (the golden model under oracle/,
 the reference itself having no CPU macroblock encoder: its encoder is Allwinner silicon,
 kernel/cedar.c:1176) on all host cores, on a bounded sample of the same workload.
+
+--dump-outputs DIR writes what the timed encode returned in its last step (see dump_outputs) for an output-for-output
+comparison of two builds: the synthetic clip depends on the arguments only.
 """
 import os
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")  # before CUDA initialises: side streams must not share queues
@@ -26,8 +29,10 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+DUMP_LIMIT = 64 << 20  # bytes that --dump-outputs writes at most
 
 WORKLOADS = {
     # name: (width, height, fmt, frames, gop, qp, me_range, cabac)
@@ -156,6 +161,24 @@ def parity_block(gops, data, sizes):
             "equal": not bad, "mismatching_gops_first_frame": bad,
             "how": "SHA-256 of the golden model's bytes for each sampled GOP == SHA-256 of the same frames of the stream "
                    "downloaded from the timed handle"}
+
+
+def dump_outputs(out_dir, stream, sizes, suffix=""):
+    """--dump-outputs: the Annex-B bytestream of the clip (float32, one value per byte) and the size of every frame in it
+    (float64), as .npy files.  A stream beyond DUMP_LIMIT is written as a fixed, seeded sample of its bytes
+    (stream_sample) with their positions (stream_sample_index)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"frame_sizes": np.asarray(sizes, np.float64)}
+    room = DUMP_LIMIT - out["frame_sizes"].nbytes - 4096  # 4096: the .npy headers
+    if 4 * len(stream) <= room:
+        out["stream"] = np.asarray(stream, np.float32)
+    else:
+        idx = np.unique(np.random.default_rng(0).integers(0, len(stream), room // 12))
+        out["stream_sample"] = np.asarray(stream[idx], np.float32)
+        out["stream_sample_index"] = idx.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def run_reference(args, rank, world):
@@ -833,6 +856,8 @@ def run_gpu(args, rank, local_rank, world):
         else:
             line["cpu_baseline"] = None
         print(json.dumps(line))
+    if args.dump_outputs:  # `data`: handle 0's stream after its last timed step (every handle's is the same bytes)
+        dump_outputs(args.dump_outputs, data, sizes, "_rank%d" % rank if world > 1 else "")
     for e in encs:
         e.close()
     if world > 1:
@@ -860,7 +885,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the other BASELINE configs and the strong-scaling clips")
     ap.add_argument("--clips-in-flight", type=int, default=0,
                     help="encoder handles per GPU, each on its own host thread; steps alternate between them (0 = 2 or 3, by --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the stream the timed encode returned in its last step to DIR/*.npy (b200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: only the b200 arm returns a whole stream")
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.impl == "reference":
         return run_reference(args, rank, world)
