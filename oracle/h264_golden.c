@@ -1650,6 +1650,7 @@ typedef struct {
     uint32_t low, range;
     int first_bit, outstanding;
     uint8_t state[1024]; /* pStateIdx << 1 | valMPS */
+    int run_max, run_carry; /* longest run of outstanding bits, and the bit that ended it (1 = a carry) */
 } cabac_t;
 
 static void cabac_init(cabac_t *c, bitw *bw, int frame_i, int qp)
@@ -1659,6 +1660,8 @@ static void cabac_init(cabac_t *c, bitw *bw, int frame_i, int qp)
     c->range = 510;
     c->first_bit = 1;
     c->outstanding = 0;
+    c->run_max = 0;
+    c->run_carry = 0;
     for (int i = 0; i < 460; i++) {
         int m = frame_i ? h264_cabac_init_I[i][0] : h264_cabac_init_P0[i][0];
         int n = frame_i ? h264_cabac_init_I[i][1] : h264_cabac_init_P0[i][1];
@@ -1672,6 +1675,10 @@ static void cabac_init(cabac_t *c, bitw *bw, int frame_i, int qp)
 
 static void cabac_put_bit(cabac_t *c, int b)
 {
+    if (c->outstanding > c->run_max) {
+        c->run_max = c->outstanding;
+        c->run_carry = b;
+    }
     if (c->first_bit)
         c->first_bit = 0;
     else
@@ -1985,6 +1992,52 @@ static void cabac_slice_data(gm_encoder *e, bitw *bw, int frame_i, int row0, int
     }
     while (bw->nbits & 7)
         bw_put(bw, 0, 1); /* rbsp_alignment_zero_bit */
+}
+
+/* One slice's RBSP from raw bins in the product's bin format (16 bits: ctxIdx in bits 0..9, 1 << 10 bypass,
+ * 1 << 11 terminate, value in bit 15): header bits, cabac_alignment_one_bits, the bins through the coder above, and
+ * the stop bit and zero padding of the final terminate(1), which must be the last bin and the only terminate(1). */
+int gm_cabac_code_bins(const uint16_t *bins, int n, int frame_i, int qp, uint64_t hdr_bits, int hdr_nbits, uint8_t *out,
+                       int cap, uint8_t *pre, int *stats)
+{
+    if (n < 1 || hdr_nbits < 0 || hdr_nbits > 64 || bins[n - 1] != (1u << 11 | 1u << 15))
+        return -EINVAL;
+    for (int i = 0; i < n; i++)
+        if ((bins[i] & 0x7000) || (bins[i] & 0x0c00) == 0x0c00 || (!(bins[i] & 0x0c00) && (bins[i] & 0x3ff) >= 460) ||
+            (i + 1 < n && bins[i] == (1u << 11 | 1u << 15)))
+            return -EINVAL;
+    bitw bw;
+    bw_init(&bw, out, (size_t)cap);
+    if (hdr_nbits > 32)
+        bw_put(&bw, (uint32_t)(hdr_bits >> 32), hdr_nbits - 32);
+    bw_put(&bw, (uint32_t)hdr_bits, hdr_nbits > 32 ? 32 : hdr_nbits);
+    while (bw.nbits & 7)
+        bw_put(&bw, 1, 1); /* cabac_alignment_one_bit */
+    const size_t data0 = bw.nbits;
+    cabac_t c;
+    cabac_init(&c, &bw, frame_i, qp);
+    for (int i = 0; i < n; i++) {
+        const int v = bins[i] >> 15;
+        if (bins[i] & (1u << 11))
+            cabac_terminate(&c, v);
+        else if (bins[i] & (1u << 10))
+            cabac_bypass(&c, v);
+        else {
+            if (pre)
+                pre[i] = c.state[bins[i] & 0x3ff];
+            cabac_decision(&c, bins[i] & 0x3ff, v);
+        }
+    }
+    if (stats) {
+        stats[0] = c.run_max;
+        stats[1] = c.run_carry;
+        stats[2] = (int)(bw.nbits - data0); /* slice data bits up to and including the stop bit */
+    }
+    while (bw.nbits & 7)
+        bw_put(&bw, 0, 1);
+    if ((bw.nbits >> 3) >= (size_t)cap) /* bw_put stops at cap */
+        return -ENOMEM;
+    return (int)(bw.nbits >> 3);
 }
 
 /* ------------------------------------------------------------------------------------------

@@ -102,6 +102,15 @@ int gm_slice_header_bits(int frame_i, int frame_p_count, int cabac, uint32_t *bi
 /* The same with first_mb_in_slice != 0 (slice_rows extension); up to 64 bits. */
 int gm_slice_header_bits64(int frame_i, int frame_p_count, int cabac, int first_mb, uint64_t *bits, int *nbits);
 
+/* The CABAC arithmetic coder on its own (for kernel-level tests of the product's coder): one slice's RBSP from the
+ * bins of the product's format (ctxIdx 0..459 in bits 0..9, 1 << 10 bypass, 1 << 11 terminate, value in bit 15; the
+ * last bin and only it is terminate(1)) coded in the initial states of (frame_i, qp) after hdr_nbits header bits.
+ * Returns the RBSP bytes written to out, -EINVAL for a malformed bin array, -ENOMEM when cap is too small.  Optional:
+ * pre[i] = the state (pStateIdx << 1 | valMPS) regular bin i was coded in; stats[0] = the longest run of outstanding
+ * bits, stats[1] = the bit that ended it (1 = a carry), stats[2] = slice data bits through the rbsp stop bit. */
+int gm_cabac_code_bins(const uint16_t *bins, int n, int frame_i, int qp, uint64_t hdr_bits, int hdr_nbits, uint8_t *out,
+                       int cap, uint8_t *pre, int *stats);
+
 /* Deterministic synthetic moving-pattern clip (integer only, stateless per pixel). */
 void gm_synth_frame(int width, int height, int format, int t, uint8_t *luma, uint8_t *chroma);
 

@@ -65,9 +65,10 @@ long hh_cavlc_slice(const void *mbi, const uint8_t *nnz, const int16_t *coef, in
     return bytes;
 }
 
-long hh_cabac_slice(const void *mbi, const uint8_t *nnz, const int16_t *coef, int mbw, int mbh, int srows, int slice,
-                    int frame_i, int qp, uint64_t hdr_bits, int hdr_nbits, uint8_t *out, long cap, int chunk_bins,
-                    const uint8_t *i4)
+// The bins of one slice (macroblock rows [row0, row1) of a picture whose slices are srows rows tall) through the
+// count / prefix-sum / write passes.  Returns the bin count; the bins are written only if they fit in cap.
+long hh_cabac_bins(const void *mbi, const uint8_t *nnz, const int16_t *coef, int mbw, int mbh, int srows, int slice,
+                   int frame_i, uint16_t *bins, long cap, const uint8_t *i4)
 {
     FrameSyntax fs{(const MbInfo *)mbi, nnz, coef, mbw, mbh, srows, i4};
     const int row0 = slice * srows, row1 = row0 + srows < mbh ? row0 + srows : mbh;
@@ -80,11 +81,22 @@ long hh_cabac_slice(const void *mbi, const uint8_t *nnz, const int16_t *coef, in
         off[i] = total;
         total += c.n;
     }
-    std::vector<uint16_t> bins(total + 1);
+    if ((long)total > cap)
+        return (long)total;
     for (int i = nmb - 1; i >= 0; i--) {
-        BinWrite w(bins.data() + off[i]);
+        BinWrite w(bins + off[i]);
         cabac_mb(w, fs, mb0 + i, frame_i);
     }
+    return (long)total;
+}
+
+// A slice's bins (ending with terminate(1)) through the serial three-stage coder and, checked against it byte for
+// byte, the parallel formulation of cabac_code_kernel emulated with chunk_bins bins per chunk.  Returns the RBSP length
+// in bytes (header bits + cabac_alignment_one_bits + slice data + stop bit, byte aligned) or a negative code.
+long hh_cabac_code_bins(const uint16_t *bins, long n, int frame_i, int qp, uint64_t hdr_bits, int hdr_nbits, uint8_t *out,
+                        long cap, int chunk_bins)
+{
+    const size_t total = (size_t)n;
     // header bits followed by cabac_alignment_one_bit up to the byte boundary
     int hb = (hdr_nbits + 7) >> 3;
     unsigned long long h = (hdr_bits << (hb * 8 - hdr_nbits)) | ((1ull << (hb * 8 - hdr_nbits)) - 1);
@@ -258,6 +270,16 @@ long hh_cabac_slice(const void *mbi, const uint8_t *nnz, const int16_t *coef, in
         out[hb + i] = v;
     }
     return hb + (long)c.pos;
+}
+
+long hh_cabac_slice(const void *mbi, const uint8_t *nnz, const int16_t *coef, int mbw, int mbh, int srows, int slice,
+                    int frame_i, int qp, uint64_t hdr_bits, int hdr_nbits, uint8_t *out, long cap, int chunk_bins,
+                    const uint8_t *i4)
+{
+    const long n = hh_cabac_bins(mbi, nnz, coef, mbw, mbh, srows, slice, frame_i, nullptr, 0, i4);
+    std::vector<uint16_t> bins(n + 1);
+    hh_cabac_bins(mbi, nnz, coef, mbw, mbh, srows, slice, frame_i, bins.data(), n, i4);
+    return hh_cabac_code_bins(bins.data(), n, frame_i, qp, hdr_bits, hdr_nbits, out, cap, chunk_bins);
 }
 
 // Emulation prevention with the order-independent rule used by the GPU kernel.

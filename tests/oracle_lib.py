@@ -71,6 +71,8 @@ def lib():
         L.gd_frame.argtypes = [C.c_void_p, C.c_int, C.c_int]
         L.gd_frame.restype = C.c_void_p
         L.gm_synth_frame.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+        L.gm_cabac_code_bins.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int, C.c_void_p, C.c_int,
+                                         C.c_void_p, C.c_void_p]
         assert C.sizeof(GmMb) == MB_DTYPE.itemsize, (C.sizeof(GmMb), MB_DTYPE.itemsize)
         _lib = L
     return _lib
@@ -176,6 +178,22 @@ def slice_header_bits(frame_i, frame_p_count, cabac, first_mb=0):
     bits, n = C.c_uint32(), C.c_int()
     lib().gm_slice_header_bits(frame_i, frame_p_count, cabac, C.byref(bits), C.byref(n))
     return format(bits.value, "0%db" % n.value)
+
+
+def cabac_code_bins(bins, frame_i, qp, hdr_bits=0, hdr_nbits=0):
+    """The golden model's spec-literal CABAC coder on raw bins (uint16, the product's bin format).  Returns
+    (rbsp bytes, pre-state of every bin (0 for bypass / terminate), (longest outstanding run, 1 if a carry ended it,
+    slice data bits through the stop bit))."""
+    bins = np.ascontiguousarray(bins, np.uint16)
+    cap = 2 * bins.size + 256
+    out = np.zeros(cap, np.uint8)
+    pre = np.zeros(bins.size, np.uint8)
+    stats = np.zeros(3, np.int32)
+    n = lib().gm_cabac_code_bins(bins.ctypes.data, bins.size, frame_i, qp, hdr_bits, hdr_nbits, out.ctypes.data, cap,
+                                 pre.ctypes.data, stats.ctypes.data)
+    if n < 0:
+        raise ValueError("gm_cabac_code_bins: %d" % n)
+    return out[:n].tobytes(), pre, tuple(int(v) for v in stats)
 
 
 def golden_decode(stream: bytes, crop=True):
