@@ -119,7 +119,7 @@ struct cedar_b200_handle {
     int16_t *d_coef[2];
     int *d_flags; // [3][L][mbh]
     uint32_t *d_me_tabs; // me_kernel's cost / task tables (me_build_tables)
-    unsigned long long *d_counters; // measurement (profiling on): [0] executed VABSDIFF4 lane-instructions, [8 + c] bins of context c
+    unsigned long long *d_counters; // measurement (profiling on): [0, 5) me_kernel (MeShape::exec_count), [8 + c] bins of context c
     bool no_prune;                  // measurement (CEDAR_B200_NO_PRUNE at open): the search accumulates every candidate to the end
     uint8_t *d_bs; // [L][nmb][32] boundary strengths
     unsigned long long *d_sse;
@@ -506,6 +506,8 @@ int encode_step(cedar_b200_handle *h, const Step &s, int t, int gop_pos0, int st
     } else {
         MeShape ms = me_shape(g.R);
         ms.noprune = h->no_prune;
+        if (h->count && h->no_prune) // the measurement without pruning: no bound either
+            ms.bound = 0;
         ms.exec_count = h->count ? h->d_counters : nullptr;
         const dim3 me_grid((g.mbw + ms.nstrip - 1) / ms.nstrip, (g.mbh + ms.nrow - 1) / ms.nrow, nl);
         const size_t me_smem = me_smem_bytes(g.R, ms.nstrip);

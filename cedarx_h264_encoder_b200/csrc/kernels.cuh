@@ -209,12 +209,38 @@ __host__ __device__ inline size_t me_smem_bytes(int R, int nstrip)
     return (size_t)(64 * nstrip * me_rows(R) + 4 * me_copy_words(R, nstrip) + me_item_words(R, nstrip)) * 4;
 }
 
+// Block-sum bound of the search (R <= 32, 4 x 4 tiles).  Split each 16 x 16 block into its sixteen 4 x 4 sub-blocks with
+// pixel sums A_g (current) and B_g (candidate).  |A - B| >= 16 |floor(A / 16) - floor(B / 16)| - 15, so
+//     SAD >= 16 * sum_g |floor(A_g / 16) - floor(B_g / 16)| - 240,
+// and the quantised sums are bytes: four VABSDIFF4 bound a candidate whose SAD takes 64.  The quantised sums of every
+// 4 x 4 window position are one table per CTA, built from the staged window; the table and the list of candidates whose
+// bound does not rule them out live in the space of the three byte-shifted window copies, which the bound path does not
+// stage (it reads copy 0 with funnel shifts).  Table row y holds four phase rows (x mod 4) of tpw words; byte b of phase
+// row c is the position x = 4 b + c, so one unaligned word of it is the four sub-block columns of a candidate.
+#define ME_LIST_CAP 2048 // candidates per tile that the SAD stage takes; a tile with more runs the exhaustive search
+__host__ __device__ inline int me_tab_pw(int R, int nstrip) { return ((16 * (nstrip - 1) + 2 * R + 12) >> 4) + 2; }
+__host__ __device__ inline int me_tab_rows(int R) { return me_window_rows(R) - 3; }
+// three more rows (zero) for the row offsets past the range that the bound stage's lanes run through
+__host__ __device__ inline int me_tab_words(int R, int nstrip) { return (me_tab_rows(R) + 3) * 4 * me_tab_pw(R, nstrip); }
+inline bool me_bound_path(int R) // the geometries that take the bound path; the rest search exhaustively
+{
+    if (R < 2 || R > 32) // R < 2: fewer than four row offsets; R > 32: 2 x 1 tiles, whose window leaves no room
+        return false;
+    const int nstrip = me_strip(R);
+    return 4 * nstrip * me_rows(R) + me_tab_words(R, nstrip) + ME_LIST_CAP <= 3 * me_copy_words(R, nstrip);
+}
+
 // Everything about the search geometry that only depends on the configuration, computed once on the host: the kernel's
 // prologue runs once per warp and 200 k warps per launch make every division in it count.
 struct MeShape {
     int nstrip, lstrip, nrow, RSW, CWs, WR, nd, nfull, nleft, ndyg; // lstrip = log2(nstrip)
+    int bound;                       // block-sum bound path (me_bound_path)
+    int tpw, trows;                  // its table: words per phase row, rows
+    uint32_t nd_magic;               // __umulhi(i, nd_magic) == i / nd for the bound stage's item indices
     int noprune;                     // measurement only (CEDAR_B200_NO_PRUNE): every candidate is accumulated to the end
-    unsigned long long *exec_count;  // measurement only (profiling on): executed VABSDIFF4 lane-instructions, else null
+    // measurement only (profiling on), else null: [0] executed VABSDIFF4 lane-instructions, [1] candidates bounded,
+    // [2] candidates that reached the SAD stage, [3] tiles on the bound path, [4] of them, tiles that searched exhaustively
+    unsigned long long *exec_count;
 };
 inline MeShape me_shape(int R)
 {
@@ -227,6 +253,10 @@ inline MeShape me_shape(int R)
     m.WR = me_window_rows(R);
     m.nd = 2 * R + 1;
     m.nfull = m.nd >> 5, m.nleft = m.nd & 31, m.ndyg = (m.nd + 3) >> 2;
+    m.bound = me_bound_path(R);
+    m.tpw = me_tab_pw(R, m.nstrip);
+    m.trows = me_tab_rows(R);
+    m.nd_magic = (uint32_t)(((1ull << 32) + (unsigned)m.nd - 1) / (unsigned)m.nd); // exact for i < 2^32 / nd
     m.noprune = 0;
     m.exec_count = nullptr;
     return m;
@@ -238,7 +268,7 @@ inline MeShape me_shape(int R)
 // kCount: the measurement build of the same kernel (profiling on): counts the executed VABSDIFF4 lane-instructions and
 // honours MeShape::noprune; the product launches kCount = false, which carries neither.
 template <int kRSW, bool kCount = false>
-__global__ void __launch_bounds__(ME_THREADS) me_kernel(Geom g, Step s, MeShape ms, const uint8_t *__restrict__ src,
+__global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, Step s, MeShape ms, const uint8_t *__restrict__ src,
                                                        const uint8_t *__restrict__ ref, MbInfo *__restrict__ mbi,
                                                        const MbInfo *__restrict__ mbi_prev,
                                                        const uint32_t *__restrict__ tabs)
@@ -247,6 +277,7 @@ __global__ void __launch_bounds__(ME_THREADS) me_kernel(Geom g, Step s, MeShape 
     __shared__ uint32_t mb_best[ME_MAX_MB];
     __shared__ uint32_t mvcost[136];      // lambda * bits(offset - R)
     __shared__ uint32_t task_tab[ME_TASK_WORDS];
+    __shared__ int list_n; // bound path: candidates that passed the bound
     if (lane_frame(s, blockIdx.z) < 0)
         return;
     const int R = g.R, nd = ms.nd, nstrip = ms.nstrip;
@@ -282,10 +313,13 @@ __global__ void __launch_bounds__(ME_THREADS) me_kernel(Geom g, Step s, MeShape 
         if ((vmask >> m) & 1)
             cur_s[i] = *(const uint32_t *)(srcY + (size_t)(y0 + 16 * (m >> ls) + row) * g.W + x0 + 16 * (m & (nstrip - 1)) + 4 * k);
     }
+    const bool bound = kRSW != 43 && ms.bound; // kRSW = 43 is R > 32, never on the bound path
+    if (tid == 0)
+        list_n = 0;
     // Window staging: warp = window row (round robin), lane = 32-bit word of the row.  Each lane fetches its
     // word and the next one (the second fetch hits L1) and builds the three byte-shifted copies in
-    // registers; no integer division, no shared-memory round trip.
-    {
+    // registers; no integer division, no shared-memory round trip.  plain: copy 0, shifted: copies 1..3.
+    auto stage = [&](const bool plain, const bool shifted) {
         const int warp_ = tid >> 5, lane_ = tid & 31;
         const bool interior_x = x0 - R >= 0 && x0 - R + 4 * RSW + 4 <= g.W && !((x0 - R) & 3);
         auto fetch = [&](const uint8_t *row, int k) -> uint32_t { // window word k of a row, edge clamped
@@ -316,10 +350,13 @@ __global__ void __launch_bounds__(ME_THREADS) me_kernel(Geom g, Step s, MeShape 
 #pragma unroll
                 for (int i = 0; i < 4; i++)
                     if (on && 4 * q + i < RSW) {
-                        d[i] = w[i];
-                        d[i + CWs] = __byte_perm(w[i], w[i + 1], 0x4321);
-                        d[i + 2 * CWs] = __byte_perm(w[i], w[i + 1], 0x5432);
-                        d[i + 3 * CWs] = __byte_perm(w[i], w[i + 1], 0x6543);
+                        if (plain)
+                            d[i] = w[i];
+                        if (shifted) {
+                            d[i + CWs] = __byte_perm(w[i], w[i + 1], 0x4321);
+                            d[i + 2 * CWs] = __byte_perm(w[i], w[i + 1], 0x5432);
+                            d[i + 3 * CWs] = __byte_perm(w[i], w[i + 1], 0x6543);
+                        }
                     }
             }
         }
@@ -333,21 +370,28 @@ __global__ void __launch_bounds__(ME_THREADS) me_kernel(Geom g, Step s, MeShape 
                     hi = fetch(row, k + 1);
                 if (k < RSW) {
                     uint32_t *d = cp + r * RSW + k;
-                    d[0] = lo;
-                    d[CWs] = __byte_perm(lo, hi, 0x4321);
-                    d[2 * CWs] = __byte_perm(lo, hi, 0x5432);
-                    d[3 * CWs] = __byte_perm(lo, hi, 0x6543);
+                    if (plain)
+                        d[0] = lo;
+                    if (shifted) {
+                        d[CWs] = __byte_perm(lo, hi, 0x4321);
+                        d[2 * CWs] = __byte_perm(lo, hi, 0x5432);
+                        d[3 * CWs] = __byte_perm(lo, hi, 0x6543);
+                    }
                 }
             }
         }
-    }
+    };
+    stage(true, !bound);
     __syncthreads();
+    // copy 0 read at byte offset ox & 3 (what copy ox & 3 holds): the seeds and the bound path's SAD stage
+    auto win = [&](const uint32_t *p, int sh) { return __funnelshift_r(p[0], p[1], sh); };
+    unsigned nabs = 0; // measurement build: VABSDIFF4 lane-instructions of the bound path
 
     const int warp = tid >> 5, lane = tid & 31, nwarps = ME_THREADS / 32;
     // Seed the running minimum with two real candidates per macroblock -- the zero vector and the vector the
     // co-located macroblock had in the previous frame (any value is fine: it only has to be a candidate of the
-    // search) -- so that the exhaustive loop below can drop a task as soon as the partial cost of every candidate
-    // in it exceeds the best complete cost so far.  SAD terms are non-negative, so the partial key is a lower
+    // search) -- so that the bound stage can reject candidates outright and the SAD loops can drop a task as soon as the
+    // partial cost of every candidate in it exceeds the best complete cost so far.  SAD terms are non-negative, so the partial key is a lower
     // bound of the final key: the argmin, and with it the bitstream, is unchanged.
     // one warp pass per macroblock: lanes 0..15 take the rows of the zero-vector seed, lanes 16..31 those of the
     // co-located one
@@ -362,17 +406,181 @@ __global__ void __launch_bounds__(ME_THREADS) me_kernel(Geom g, Step s, MeShape 
             oy = clip3_(0, nd - 1, (pv.mv[1] >> 2) + R);
         }
         uint32_t a = 0;
-        const uint32_t *wp = cp + (ox & 3) * CWs + (oy + 16 * mr + l16) * RSW + 4 * mc + (ox >> 2);
+        const uint32_t *wp = cp + (oy + 16 * mr + l16) * RSW + 4 * mc + (ox >> 2);
         const uint32_t *cu = cur_s + 64 * m + 4 * l16;
 #pragma unroll
         for (int k = 0; k < 4; k++)
-            a = sad4_acc(wp[k], cu[k], a);
+            a = sad4_acc(win(wp + k, 8 * (ox & 3)), cu[k], a);
         a = __reduce_add_sync(half ? 0xffff0000u : 0x0000ffffu, a);
         if (l16 == 0)
             atomicMin(&mb_best[m], ((a + mvcost[ox] + mvcost[oy]) << 15) | (uint32_t)(oy * nd + ox));
     }
+    // Bound path: the quantised 4 x 4 sums of the current blocks (word 4 m + i = sub-block row i of macroblock m, byte j =
+    // sub-block column j) and of every window position (tab, see me_tab_pw)
+    uint32_t *const qcur = cp + CWs, *const tab = qcur + 4 * nmb, *const list = tab + (ms.trows + 3) * 4 * ms.tpw;
+    const int tpw = ms.tpw, tw = 4 * tpw;
+    if (bound) {
+        if (tid < 4 * nmb && ((vmask >> (tid >> 2)) & 1)) {
+            const uint32_t *cu = cur_s + 16 * tid;
+            uint32_t q = 0;
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                uint32_t a = 0;
+#pragma unroll
+                for (int r = 0; r < 4; r++)
+                    a = sad4_acc(cu[4 * r + j], 0u, a);
+                q |= (a >> 4) << (8 * j);
+            }
+            qcur[tid] = q;
+            if (kCount)
+                nabs += 16;
+        }
+        for (int i = tid; i < 3 * tw; i += ME_THREADS)
+            tab[ms.trows * tw + i] = 0;
+        // thread = (segment of kSeg table rows, phase c, word w): four running rows of 4-pixel sums per column, so every
+        // window word is read once per segment.  Bytes of positions no candidate reaches are 0.
+        constexpr int kSeg = 12;
+        const int xs_max = 16 * (nstrip - 1) + 2 * R + 12, nseg = (ms.trows + kSeg - 1) / kSeg;
+        for (int it = tid; it < nseg * tw; it += ME_THREADS) {
+            const int seg = it / tw, col = it - seg * tw, c = col / tpw, w = col - c * tpw;
+            const int y0 = seg * kSeg, y1 = imin_(y0 + kSeg, ms.trows), sh = 8 * c;
+            int idx[4];
+            uint32_t valid = 0;
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                idx[j] = imin_(4 * w + j, RSW - 2);
+                valid |= (16 * w + c + 4 * j <= xs_max ? 0xffu : 0u) << (8 * j);
+            }
+            auto hrow = [&](int y, uint32_t *hh) {
+#pragma unroll
+                for (int j = 0; j < 4; j++)
+                    hh[j] = sad4_acc(win(cp + y * RSW + idx[j], sh), 0u, 0u);
+            };
+            auto put = [&](int y, const uint32_t *a, const uint32_t *b, const uint32_t *c_, const uint32_t *d) {
+                uint32_t q = 0;
+#pragma unroll
+                for (int j = 0; j < 4; j++)
+                    q |= ((a[j] + b[j] + c_[j] + d[j]) >> 4) << (8 * j);
+                tab[y * tw + col] = q & valid;
+            };
+            uint32_t h0[4], h1[4], h2[4], h3[4];
+            hrow(y0, h0), hrow(y0 + 1, h1), hrow(y0 + 2, h2);
+            for (int y = y0; y < y1; y += 4) {
+                hrow(y + 3, h3), put(y, h0, h1, h2, h3);
+                if (y + 1 < y1)
+                    hrow(y + 4, h0), put(y + 1, h1, h2, h3, h0);
+                if (y + 2 < y1)
+                    hrow(y + 5, h1), put(y + 2, h2, h3, h0, h1);
+                if (y + 3 < y1)
+                    hrow(y + 6, h2), put(y + 3, h3, h0, h1, h2);
+            }
+            if (kCount)
+                nabs += 4 * (y1 - y0 + 3);
+        }
+    }
     __syncthreads();
-    const int ntask = ntask_full * nmb + ((nitems_left + 31) >> 5);
+    bool fallback = !bound;
+    unsigned nbounded = 0, nsad = 0; // measurement build
+    if (bound) {
+        // Bound stage: item = (macroblock m, row phase c, column offset ox); a lane walks the row offsets c, c + 4, ..
+        // and keeps the three table rows the next candidate shares.  A candidate whose bound key exceeds the best key
+        // of the seeds cannot be the argmin (its key is at least the bound key); the others go to the list.
+        const int nitem = nmb * 4 * nd;
+        for (int i0 = warp * 32; i0 < nitem; i0 += nwarps * 32) {
+            if (__shfl_sync(0xffffffffu, *(volatile int *)&list_n, 0) > ME_LIST_CAP)
+                break; // the tile searches exhaustively: no need to bound the rest
+            const int i = i0 + lane, t = (int)__umulhi((uint32_t)i, ms.nd_magic), ox = i - t * nd, c = t & 3;
+            const bool live = i < nitem && ((vmask >> (t >> 2)) & 1);
+            const int m = live ? t >> 2 : 0, x = 16 * (m & (nstrip - 1)) + ox, sh = 8 * ((x >> 2) & 3);
+            // no branch per candidate: every lane runs ndyg row offsets (the table has rows for the ones past the range,
+            // whose results are masked off) and sets bit j of pm when row offset c + 4 j passes
+            const uint32_t *tp = tab + (16 * (m >> ls) + c) * tw + (x & 3) * tpw + (x >> 4);
+            const uint4 q = ((const uint4 *)qcur)[m];
+            const uint32_t best = mb_best[m], cx = mvcost[ox] - 240u; // cost = max(16 sb, 240) - 240 + mv cost
+            uint32_t w0 = win(tp, sh), w1 = win(tp + 4 * tw, sh), w2 = win(tp + 8 * tw, sh), pm = 0;
+            uint32_t rank = (uint32_t)(c * nd + ox);
+            for (int j = 0; j < ndyg; j++) {
+                const uint32_t w3 = win(tp + (4 * j + 12) * tw, sh);
+                uint32_t sb = sad4_acc(w0, q.x, 0u);
+                sb = sad4_acc(w1, q.y, sb);
+                sb = sad4_acc(w2, q.z, sb);
+                sb = sad4_acc(w3, q.w, sb);
+                const uint32_t key = (max(16u * sb, 240u) + cx + mvcost[c + 4 * j]) * 32768u + rank;
+                pm |= (uint32_t)(key <= best) << j;
+                rank += 4u * (uint32_t)nd;
+                w0 = w1, w1 = w2, w2 = w3;
+            }
+            pm &= live ? (1u << ((nd - c + 3) >> 2)) - 1u : 0u; // row offsets c + 4 j < nd
+            if (kCount && live)
+                nbounded += (nd - c + 3) >> 2;
+            // append the passing candidates: one ballot and one shared atomic per round, a round per set bit
+            while (__any_sync(0xffffffffu, pm)) {
+                const bool pass = pm != 0;
+                const int oy = c + 4 * (__ffs(pm) - 1);
+                pm &= pm - 1;
+                const uint32_t ball = __ballot_sync(0xffffffffu, pass);
+                int base = 0;
+                if (lane == 0)
+                    base = atomicAdd(&list_n, __popc(ball));
+                base = __shfl_sync(0xffffffffu, base, 0) + __popc(ball & ((1u << lane) - 1));
+                if (pass && base < ME_LIST_CAP)
+                    list[base] = (uint32_t)m | ((uint32_t)ox << 4) | ((uint32_t)oy << 12);
+            }
+        }
+        if (kCount)
+            nabs += 4 * nbounded;
+        __syncthreads();
+        fallback = list_n > ME_LIST_CAP;
+        if (!fallback) {
+            // SAD stage: one listed candidate per thread, read from copy 0, with a partial-cost exit after eight rows
+            const int n = list_n;
+            for (int i = tid; i < n; i += ME_THREADS) {
+                const uint32_t e = list[i];
+                const int m = (int)(e & 15), ox = (int)((e >> 4) & 255), oy = (int)(e >> 12), sh = 8 * (ox & 3);
+                const uint32_t *wp = cp + (oy + 16 * (m >> ls)) * RSW + 4 * (m & (nstrip - 1)) + (ox >> 2);
+                const uint4 *cu = (const uint4 *)(cur_s + 64 * m);
+                const uint32_t rank = (uint32_t)(oy * nd + ox);
+                uint32_t acc = mvcost[ox] + mvcost[oy];
+                bool dead = false;
+#pragma unroll
+                for (int r = 0; r < 16; r++) {
+                    if (r == 8) {
+                        dead = ((acc << 15) | rank) > *(volatile uint32_t *)&mb_best[m];
+                        if (dead)
+                            break;
+                    }
+                    const uint4 cw = cu[r];
+                    const uint32_t *p = wp + r * RSW;
+                    acc = sad4_acc(win(p, sh), cw.x, acc);
+                    acc = sad4_acc(win(p + 1, sh), cw.y, acc);
+                    acc = sad4_acc(win(p + 2, sh), cw.z, acc);
+                    acc = sad4_acc(win(p + 3, sh), cw.w, acc);
+                }
+                if (kCount)
+                    nabs += dead ? 32 : 64, nsad++;
+                if (!dead)
+                    atomicMin(&mb_best[m], (acc << 15) | rank);
+            }
+        } else {
+            stage(false, true); // the exhaustive search below reads the byte-shifted copies
+            __syncthreads();
+        }
+    }
+    if (kCount && ms.exec_count && bound) {
+        const unsigned a = __reduce_add_sync(0xffffffffu, nabs), b = __reduce_add_sync(0xffffffffu, nbounded),
+                       c = __reduce_add_sync(0xffffffffu, nsad);
+        if (lane == 0) {
+            atomicAdd(ms.exec_count, (unsigned long long)a);
+            atomicAdd(ms.exec_count + 1, (unsigned long long)b);
+            atomicAdd(ms.exec_count + 2, (unsigned long long)c);
+        }
+        if (tid == 0) {
+            atomicAdd(ms.exec_count + 3, 1ull);
+            atomicAdd(ms.exec_count + 4, (unsigned long long)fallback);
+        }
+    }
+    // Exhaustive search: every geometry off the bound path, and bound-path tiles whose list overflowed
+    const int ntask = fallback ? ntask_full * nmb + ((nitems_left + 31) >> 5) : 0;
     for (int task = warp; task < ntask; task += nwarps) {
         // task table entry: macroblock | column offset << 4 | first row offset << 12 (0xffffffff = idle lane)
         const uint32_t e = task < ntask_full * nmb ? task_tab[task] + ((uint32_t)lane << 4)
