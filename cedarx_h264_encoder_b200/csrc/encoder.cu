@@ -12,6 +12,7 @@
 
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -78,17 +79,13 @@ struct cedar_b200_handle {
     cudaEvent_t ev_ingest[2], ev_main[2], ev_post[2], ev_begin, ev_post_done;
     cudaEvent_t ev_syn[2], ev_ent[2]; // syntax records of step parity p final (after bs_kernel) / its entropy passes done
     bool post_valid[2]; // ev_post[p] has been recorded in this stream of work
-    // clip upload: host->device copies run on their own stream in step order; step t waits for ev_upload[t] only
+    // Clip upload, paced: clip_upload only notes the request; clip_encode issues the host->device copies of pass j + 1 on
+    // stream_copy behind the ingest of pass j, and pass j waits for ev_upload[j] only.  One pass ahead keeps the least of
+    // this handle queued on the copy engine, which serves copies in issue order; it measured best (DESIGN.md 4).
     cudaStream_t stream_copy;
     std::vector<cudaEvent_t> ev_upload;
     cudaEvent_t ev_encode_done;
-    bool upload_pending;
-    // Paced upload (D = CEDAR_B200_UPLOAD_AHEAD, default 1): clip_upload only notes the request; clip_encode issues the
-    // copies of pass j + D behind the ingest of pass j, so that at most D passes of this handle are queued on the copy
-    // engine and the first frames of another handle's next clip are not stuck behind a whole clip of copies (the copy
-    // engine serves copies in issue order).  Measured, three handles, 1080p end to end: D = 0 (all copies at once)
-    // 12 050-12 600 frames/s, D = 1 13 000-13 700, D = 2 12 660-12 770, D = 8 12 720; device resident 14 000.
-    int upload_ahead, upload_deferred_n;
+    int upload_n; // frames of the last clip_upload whose copies are not issued yet, 0 for none
     cudaEvent_t ev_cabac[NSIDE];
     unsigned side_used; // bit i: side stream i has work the main stream has not joined yet
     int side_next;
@@ -365,12 +362,11 @@ int alloc_entropy_buffers(cedar_b200_handle *h)
     return r;
 }
 
-int alloc_buffers(cedar_b200_handle *h)
+// Frame-mode I/O (struct cedar_b200_io), sized like cedar_buffers_init (cedar.c:610-624) but in pinned host memory.
+int alloc_frame_io(cedar_b200_handle *h)
 {
     const Geom &g = h->g;
-    const int F = h->F, L = h->L;
     int r = 0;
-    // frame-mode I/O, sized like cedar_buffers_init (cedar.c:610-624) but in pinned host memory
     h->in_luma_size = (int)ALIGN_UP((size_t)g.src_w * g.src_h, 4096);
     size_t chroma_bytes = (size_t)g.src_w * g.src_h / (g.src_format == CEDAR_B200_FORMAT_NV16 ? 1 : 2);
     h->in_chroma_size = (int)ALIGN_UP(chroma_bytes, 4096);
@@ -378,6 +374,24 @@ int alloc_buffers(cedar_b200_handle *h)
     r |= hmalloc(&h->h_in_luma, h->in_luma_size);
     r |= hmalloc(&h->h_in_chroma, h->in_chroma_size);
     r |= hmalloc(&h->h_bytestream, h->bytestream_size);
+    return r;
+}
+
+void fill_io(const cedar_b200_handle *h, cedar_b200_io *io)
+{
+    io->input_luma = h->h_in_luma;
+    io->input_luma_size = h->in_luma_size;
+    io->input_chroma = h->h_in_chroma;
+    io->input_chroma_size = h->in_chroma_size;
+    io->bytestream = h->h_bytestream;
+    io->bytestream_size = h->bytestream_size;
+}
+
+int alloc_buffers(cedar_b200_handle *h)
+{
+    const Geom &g = h->g;
+    const int F = h->F, L = h->L;
+    int r = alloc_frame_io(h);
     r |= hmalloc(&h->h_frame_bytes, F);
     r |= hmalloc(&h->h_total, 1);
     r |= hmalloc(&h->h_sse, F);
@@ -458,6 +472,41 @@ void free_buffers(cedar_b200_handle *h)
             cudaFreeHost(p);
 }
 
+// The streams of a step's ingest, entropy / SSE passes and CABAC coders.  Profile modes 2 and 3 (h->serialize) put
+// everything on the main stream instead, so that per-kernel event times are standalone times.
+struct StepStreams {
+    cudaStream_t pre, post, side;
+};
+StepStreams step_streams(const cedar_b200_handle *h)
+{
+    if (h->serialize)
+        return {h->stream, h->stream, h->stream};
+    return {h->stream_pre, h->stream_post, h->stream_cabac[h->side_next]};
+}
+
+// The instantiation of me_kernel for a search shape: the row strides of the 1080p (R = 16: 27 words) and 4K (R = 64: 43
+// words) geometries are compiled in, and serve every range with the same stride; the rest run the generic build.
+// count: the measurement build (executed-instruction counter, CEDAR_B200_NO_PRUNE).
+decltype(&me_kernel<0>) me_kernel_for(int RSW, bool count)
+{
+    switch (RSW) {
+    case 27: return count ? me_kernel<27, true> : me_kernel<27>;
+    case 43: return count ? me_kernel<43, true> : me_kernel<43>;
+    default: return count ? me_kernel<0, true> : me_kernel<0>;
+    }
+}
+
+// The dynamic shared memory ceiling of every me_kernel instantiation: the most that any search range validate() admits
+// needs.  The ceiling belongs to the kernel on the device, not to a handle, so one that depended on the handle's range
+// would be lowered under a live handle by the open() of another one with a smaller range.
+int me_smem_ceiling()
+{
+    size_t m = 0;
+    for (int R = 1; R <= 64; R++)
+        m = std::max(m, me_smem_bytes(R, me_strip(R)));
+    return (int)m;
+}
+
 // One lock-step pass over s.nlanes lanes (one frame per lane).  t = position inside the GOP (0 => IDR).
 //   stream_pre : ingest(t)                                   -> src[p]                 (p = step parity)
 //   stream     : intra | ME, residual, MVP/skip; bS; deblock -> syntax[p], unf, rec[t & 1]
@@ -465,12 +514,6 @@ void free_buffers(cedar_b200_handle *h)
 //                                                            -> RBSP (CAVLC) or bins (CABAC)
 //   side stream: cabac_resolve_kernel, cabac_code_kernel
 // Buffers with index p are reused two steps later, hence the waits on ev_post[p].
-static bool no_overlap_env()
-{
-    static const bool v = getenv("CEDAR_B200_NO_OVERLAP") != nullptr;
-    return v;
-}
-
 int encode_step(cedar_b200_handle *h, const Step &s, int t, int gop_pos0, int step_index, bool wait_upload)
 {
     const Geom &g = h->g;
@@ -481,14 +524,14 @@ int encode_step(cedar_b200_handle *h, const Step &s, int t, int gop_pos0, int st
     MbInfo *mbi = h->d_mbi[p];
     uint8_t *nnz = h->d_nnz[p], *bs = h->d_bs;
     int16_t *coef = h->d_coef[p];
-    const bool no_overlap = no_overlap_env() || h->serialize; // diagnosis / per-kernel timing: everything in line
-    cudaStream_t st = h->stream, pre = no_overlap ? st : h->stream_pre, post = no_overlap ? st : h->stream_post;
+    const StepStreams ss = step_streams(h);
+    cudaStream_t st = h->stream, pre = ss.pre, post = ss.post;
 
     // ---- one step ahead: ingest ----
     if (h->post_valid[p])
         CK(cudaStreamWaitEvent(pre, h->ev_post[p], 0)); // step - 2 has finished with src[p] (and main with it)
     if (wait_upload)
-        CK(cudaStreamWaitEvent(pre, h->ev_upload[h->upload_deferred_n ? step_index : t], 0));
+        CK(cudaStreamWaitEvent(pre, h->ev_upload[step_index], 0));
     LAUNCH_ON(pre, K_INGEST, ingest_kernel, dim3((unsigned)((g.W / 16 + 127) / 128), (unsigned)(g.H + 2 * g.CH), nl), 128, 0, g, s, h->d_raw,
               h->raw_frame_bytes, src);
     CK(cudaEventRecord(h->ev_ingest[p], pre));
@@ -511,23 +554,8 @@ int encode_step(cedar_b200_handle *h, const Step &s, int t, int gop_pos0, int st
         ms.exec_count = h->count ? h->d_counters : nullptr;
         const dim3 me_grid((g.mbw + ms.nstrip - 1) / ms.nstrip, (g.mbh + ms.nrow - 1) / ms.nrow, nl);
         const size_t me_smem = me_smem_bytes(g.R, ms.nstrip);
-        // the 1080p (R = 16) and 4K (R = 64) geometries have compiled-in row strides
-#define ME_LAUNCH(RSW_, COUNT_)                                                                                          \
-    LAUNCH_ON(st, K_ME, (me_kernel<RSW_, COUNT_>), me_grid, ME_THREADS, me_smem, g, s, ms, src, ref, mbi, h->d_mbi[p ^ 1], h->d_me_tabs)
-        if (h->count) { // the measurement build (executed-instruction counter, CEDAR_B200_NO_PRUNE)
-            switch (ms.RSW) {
-            case 27: ME_LAUNCH(27, true); break;
-            case 43: ME_LAUNCH(43, true); break;
-            default: ME_LAUNCH(0, true); break;
-            }
-        } else {
-            switch (ms.RSW) {
-            case 27: ME_LAUNCH(27, false); break;
-            case 43: ME_LAUNCH(43, false); break;
-            default: ME_LAUNCH(0, false); break;
-            }
-        }
-#undef ME_LAUNCH
+        const auto me = me_kernel_for(ms.RSW, h->count);
+        LAUNCH_ON(st, K_ME, me, me_grid, ME_THREADS, me_smem, g, s, ms, src, ref, mbi, h->d_mbi[p ^ 1], h->d_me_tabs);
         LAUNCH_ON(st, K_INTER, inter_kernel, dim3((g.nmb + 3) / 4, nl), 128, 0, g, s, src, ref, unf, mbi, nnz, coef);
         if (g.p_intra) { // decide (parallel), then re-code the chosen macroblocks as intra in wavefront order
             CK(cudaMemsetAsync(h->d_pcount, 0, sizeof(int) * h->L, st));
@@ -565,14 +593,13 @@ int encode_step(cedar_b200_handle *h, const Step &s, int t, int gop_pos0, int st
     h->post_valid[p] = true;
     if (g.cabac) {
         // the bins of these frames are final: code them on a side stream while the next frames are reconstructed
-        cudaStream_t side = no_overlap ? st : h->stream_cabac[h->side_next];
-        CK(cudaStreamWaitEvent(side, h->ev_ent[p], 0));
-        LAUNCH_ON(side, K_CRESOLVE, cabac_resolve_kernel, nl * g.nslices, RES_THREADS, RES_SMEM_BYTES, g, s, h->K, gop_pos0, h->eb,
+        CK(cudaStreamWaitEvent(ss.side, h->ev_ent[p], 0));
+        LAUNCH_ON(ss.side, K_CRESOLVE, cabac_resolve_kernel, nl * g.nslices, RES_THREADS, RES_SMEM_BYTES, g, s, h->K, gop_pos0, h->eb,
                   h->count ? h->d_counters + 8 : nullptr);
         EntropyBufs ebc = h->eb; // the limb scratch of this side stream (its launches are serialised)
-        ebc.limbs += (size_t)(no_overlap || !h->clip_mode ? 0 : h->side_next) * h->L * g.nslices * h->eb.limb_cap;
-        LAUNCH_ON(side, K_CCODE, cabac_code_kernel, nl * g.nslices, CP_THREADS, CP_SMEM_BYTES, g, s, ebc);
-        if (!no_overlap) {
+        ebc.limbs += (size_t)(h->serialize || !h->clip_mode ? 0 : h->side_next) * h->L * g.nslices * h->eb.limb_cap;
+        LAUNCH_ON(ss.side, K_CCODE, cabac_code_kernel, nl * g.nslices, CP_THREADS, CP_SMEM_BYTES, g, s, ebc);
+        if (!h->serialize) {
             h->side_used |= 1u << h->side_next;
             h->side_next = (h->side_next + 1) % cedar_b200_handle::NSIDE;
         }
@@ -647,6 +674,16 @@ int begin_stream(cedar_b200_handle *h, int nframes)
     CK(cudaStreamWaitEvent(h->stream_post, h->ev_begin, 0));
     h->post_valid[0] = h->post_valid[1] = false;
     return 0;
+}
+
+// The frame-mode counters after a frame, cedar.c:1193-1196 (the reference swap of :1198-1201 is the `t & 1` buffer choice
+// in encode_step).
+void count_frame(cedar_b200_handle *h)
+{
+    h->frame_p_count++;
+    if (h->frame_p_count == h->K)
+        h->frame_p_count = 0;
+    h->frame_count++;
 }
 
 int check_error(cedar_b200_handle *h)
@@ -730,24 +767,12 @@ static int open_queued(const struct cedar_b200_config *cfg, struct cedar_b200_io
     int r = cedar_b200_pipe_open(&wc, nullptr, 0, 2, cfg->queue_gops, &h->pipe);
     if (r)
         return r;
-    const Geom &g = h->g;
-    h->in_luma_size = (int)ALIGN_UP((size_t)g.src_w * g.src_h, 4096);
-    size_t chroma_bytes = (size_t)g.src_w * g.src_h / (g.src_format == CEDAR_B200_FORMAT_NV16 ? 1 : 2);
-    h->in_chroma_size = (int)ALIGN_UP(chroma_bytes, 4096);
-    h->bytestream_size = (int)ALIGN_UP((size_t)g.nmb * 1536 + 4096, 4096);
-    r |= hmalloc(&h->h_in_luma, h->in_luma_size);
-    r |= hmalloc(&h->h_in_chroma, h->in_chroma_size);
-    r |= hmalloc(&h->h_bytestream, h->bytestream_size);
+    r = alloc_frame_io(h);
     r |= hmalloc(&h->h_sse, 1);
     if (r)
         return r;
     h->q_cap = cfg->queue_gops * h->K;
-    io->input_luma = h->h_in_luma;
-    io->input_luma_size = h->in_luma_size;
-    io->input_chroma = h->h_in_chroma;
-    io->input_chroma_size = h->in_chroma_size;
-    io->bytestream = h->h_bytestream;
-    io->bytestream_size = h->bytestream_size;
+    fill_io(h, io);
     return 0;
 }
 
@@ -833,13 +858,6 @@ int cedar_b200_open(const struct cedar_b200_config *cfg, struct cedar_b200_io *i
     for (int i = 0; ok && i < 2; i++)
         ok = mkevent(&h->ev_ingest[i]) && mkevent(&h->ev_main[i]) && mkevent(&h->ev_post[i]) && mkevent(&h->ev_syn[i]) &&
              mkevent(&h->ev_ent[i]);
-    {
-        const char *ua = getenv("CEDAR_B200_UPLOAD_AHEAD");
-        h->upload_ahead = ua ? atoi(ua) : 1;
-        if (h->upload_ahead < 0)
-            h->upload_ahead = 0;
-        h->upload_deferred_n = 0;
-    }
     // one event per pass of the longest clip: K passes per wave of L GOPs
     h->ev_upload.assign(h->clip_mode ? (size_t)h->K * (size_t)(((h->F + h->K - 1) / h->K + h->L - 1) / h->L) : 0, nullptr);
     for (auto &e : h->ev_upload)
@@ -858,14 +876,13 @@ int cedar_b200_open(const struct cedar_b200_config *cfg, struct cedar_b200_io *i
         destroy_handle(h);
         return -ENODEV;
     }
-    const int me_smem = (int)me_smem_bytes(g.R, me_strip(g.R));
-    if (cudaFuncSetAttribute(me_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) != cudaSuccess ||
-        cudaFuncSetAttribute(me_kernel<27>, cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) != cudaSuccess ||
-        cudaFuncSetAttribute(me_kernel<43>, cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) != cudaSuccess ||
-        cudaFuncSetAttribute(me_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) != cudaSuccess ||
-        cudaFuncSetAttribute(me_kernel<27, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) != cudaSuccess ||
-        cudaFuncSetAttribute(me_kernel<43, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) != cudaSuccess) {
-        fprintf(stderr, "cedar_b200: search range %d needs more shared memory than the device offers\n", g.R);
+    const int me_smem = me_smem_ceiling(); // the same for every handle: concurrent opens agree
+    for (int rsw : {0, 27, 43}) // every instantiation
+        for (bool count : {false, true})
+            ok = ok && cudaFuncSetAttribute(me_kernel_for(rsw, count), cudaFuncAttributeMaxDynamicSharedMemorySize, me_smem) ==
+                           cudaSuccess;
+    if (!ok) {
+        fprintf(stderr, "cedar_b200: me_kernel needs %d bytes of dynamic shared memory, more than the device offers\n", me_smem);
         cudaGetLastError();
         destroy_handle(h);
         return -EINVAL;
@@ -888,12 +905,7 @@ int cedar_b200_open(const struct cedar_b200_config *cfg, struct cedar_b200_io *i
         return r;
     }
     h->prefix_len = n1 + n2;
-    io->input_luma = h->h_in_luma;
-    io->input_luma_size = h->in_luma_size;
-    io->input_chroma = h->h_in_chroma;
-    io->input_chroma_size = h->in_chroma_size;
-    io->bytestream = h->h_bytestream;
-    io->bytestream_size = h->bytestream_size;
+    fill_io(h, io);
     *out = h;
     return 0;
 }
@@ -956,11 +968,7 @@ static int queued_encode_frame(cedar_b200_handle *h)
         if (r)
             return r;
     }
-    // cedar.c:1193-1196
-    h->frame_p_count++;
-    if (h->frame_p_count == h->K)
-        h->frame_p_count = 0;
-    h->frame_count++;
+    count_frame(h);
     return ret;
 }
 
@@ -1023,11 +1031,7 @@ int cedar_b200_encode_frame(cedar_b200_handle *h)
     CK(cudaStreamSynchronize(h->stream));
     h->last_nframes = 1;
     h->sse_valid = true;
-    // cedar.c:1193-1196 (the reference swap of :1198-1201 is the `t & 1` buffer choice in encode_step)
-    h->frame_p_count++;
-    if (h->frame_p_count == h->K)
-        h->frame_p_count = 0;
-    h->frame_count++;
+    count_frame(h);
     h->busy_ns += std::chrono::duration<double, std::nano>(std::chrono::steady_clock::now() - t0).count();
     return (int)total;
 }
@@ -1045,33 +1049,12 @@ int cedar_b200_clip_upload(cedar_b200_handle *h, int nframes)
 {
     if (!h || !h->h_clip_in || nframes <= 0 || nframes > h->F)
         return -EINVAL;
-    cudaSetDevice(h->device);
-    if (h->upload_ahead > 0) { // paced: the copies are issued by the clip_encode that follows (upload_pass)
-        h->upload_deferred_n = nframes;
-        h->upload_pending = true;
-        return 0;
-    }
-    h->upload_deferred_n = 0;
-    // Copies are issued in the order the encoder consumes the frames (step t needs frame t of every GOP) on a
-    // dedicated stream; clip_encode's step t waits for ev_upload[t] only, so the transfer overlaps the encode.
-    CK(cudaEventRecord(h->ev_encode_done, h->stream)); // do not overwrite frames a running encode still reads
-    CK(cudaStreamWaitEvent(h->stream_copy, h->ev_encode_done, 0));
-    const int K = h->K, gops = (nframes + K - 1) / K;
-    const size_t fb = h->raw_frame_bytes;
-    for (int t = 0; t < K; t++) {
-        for (int gp = 0; gp < gops; gp++) {
-            size_t f = (size_t)gp * K + t;
-            if (f < (size_t)nframes)
-                CK(cudaMemcpyAsync(h->d_raw + f * fb, h->h_clip_in + f * fb, fb, cudaMemcpyHostToDevice, h->stream_copy));
-        }
-        CK(cudaEventRecord(h->ev_upload[t], h->stream_copy));
-    }
-    h->upload_pending = true;
+    h->upload_n = nframes; // the clip_encode that follows issues the copies (upload_pass)
     return 0;
 }
 
 // Paced upload: the host -> device copies of pass j (frame t = j % K of the GOPs of wave j / K) on the copy stream, behind
-// `gate` (an event of the pass `upload_ahead` passes earlier); ev_upload[j] tells the pass that its frames are resident.
+// `gate` (an event of the pass before); ev_upload[j] tells the pass that its frames are resident.
 static int upload_pass(cedar_b200_handle *h, int nframes, int j, cudaEvent_t gate)
 {
     const int K = h->K, gops = (nframes + K - 1) / K, t = j % K, gop0 = (j / K) * h->L;
@@ -1096,43 +1079,38 @@ static int run_clip(cedar_b200_handle *h, int nframes, int first_frame_index)
     h->eb.hdr_nbits = h->d_hdr_nbits;
     if ((r = begin_stream(h, nframes)))
         return r;
-    const int K = h->K, gops = (nframes + K - 1) / K;
-    const bool paced = h->upload_pending && h->upload_deferred_n > 0;
-    const int up_n = h->upload_deferred_n, D = h->upload_ahead;
-    if (paced) {
-        // the first D passes: as soon as no earlier ingest reads d_raw any more (all of them are on stream_pre)
-        CK(cudaEventRecord(h->ev_encode_done, (h->serialize || no_overlap_env()) ? h->stream : h->stream_pre));
-        for (int j = 0; j < D; j++)
-            if ((r = upload_pass(h, up_n, j, h->ev_encode_done)))
-                return r;
+    const int K = h->K, gops = (nframes + K - 1) / K, up_n = h->upload_n;
+    const cudaStream_t pre = step_streams(h).pre;
+    if (up_n) {
+        // pass 0: as soon as no earlier ingest reads d_raw any more (all of them are on the pre stream)
+        CK(cudaEventRecord(h->ev_encode_done, pre));
+        if ((r = upload_pass(h, up_n, 0, h->ev_encode_done)))
+            return r;
     }
-    int step_index = 0;
+    int j = 0; // pass: wave gop0 / L, position t (upload_pass numbers them the same way)
     for (int gop0 = 0; gop0 < gops; gop0 += h->L) {
         int nl = gops - gop0 < h->L ? gops - gop0 : h->L;
         for (int t = 0; t < K; t++) {
             Step s = {nl, gop0 * K + t, K, nframes};
             if (s.frame0 >= nframes)
                 break;
-            if (paced && step_index != (gop0 / h->L) * K + t)
-                return -EIO; // pass numbering of upload_pass and of this loop must agree
-            if ((r = encode_step(h, s, t, 0, step_index, h->upload_pending)))
+            j = (gop0 / h->L) * K + t;
+            if ((r = encode_step(h, s, t, 0, j, up_n > 0)))
                 return r;
-            if (paced && (r = upload_pass(h, up_n, step_index + D, h->ev_ingest[step_index & 1])))
+            if (up_n && (r = upload_pass(h, up_n, j + 1, h->ev_ingest[j & 1])))
                 return r;
-            step_index++;
         }
     }
-    if (paced && up_n > nframes) { // a clip_upload of more frames than this encode covers: the rest of it now, and
-                                   // every later ingest behind it (nothing else would wait for these copies)
+    if (up_n > nframes) { // a clip_upload of more frames than this encode covers: the rest of it (past pass j + 1) now,
+                          // and every later ingest behind it (nothing else would wait for these copies)
         const int last = (int)h->ev_upload.size() - 1;
-        for (int j = step_index + D; j <= last; j++)
-            if ((r = upload_pass(h, up_n, j, h->ev_ingest[(step_index - 1) & 1])))
+        for (int k = j + 2; k <= last; k++)
+            if ((r = upload_pass(h, up_n, k, h->ev_ingest[j & 1])))
                 return r;
         CK(cudaEventRecord(h->ev_upload[last], h->stream_copy));
-        CK(cudaStreamWaitEvent((h->serialize || no_overlap_env()) ? h->stream : h->stream_pre, h->ev_upload[last], 0));
+        CK(cudaStreamWaitEvent(pre, h->ev_upload[last], 0));
     }
-    h->upload_pending = false;
-    h->upload_deferred_n = 0;
+    h->upload_n = 0;
     return finish_stream(h, nframes, 0, first_frame_index == 0);
 }
 

@@ -120,10 +120,9 @@ void cedar_b200_close(cedar_b200_handle *h);
 void *cedar_b200_clip_input(cedar_b200_handle *h, size_t *frame_bytes);
 
 /* Host -> device copy of the first nframes of the staging area.  Asynchronous, and paced by the encode that follows:
- * the copies of a pass are issued by cedar_b200_clip_encode, one pass ahead of the pass that consumes them (so that
- * several handles share the copy engine frame by frame, not clip by clip; CEDAR_B200_UPLOAD_AHEAD=0 in the environment
- * at open() issues all copies here instead).  Either way the staging area must not be written again before the
- * cedar_b200_clip_download (or cedar_b200_stats) of that encode has returned. */
+ * the copies of a pass are issued by cedar_b200_clip_encode, one pass ahead of the pass that consumes them, so that
+ * several handles share the copy engine frame by frame, not clip by clip.  The staging area must not be written again
+ * before the cedar_b200_clip_download (or cedar_b200_stats) of that encode has returned. */
 int cedar_b200_clip_upload(cedar_b200_handle *h, int nframes);
 
 /* Encode nframes already resident in device memory; frame `first_frame_index + i` of the stream

@@ -11,7 +11,7 @@ benchmark clip (1920x1080 NV12, 600 frames, GOP 60, QP 25), the step body varied
   encode+download   clip_encode + clip_download (waits, 10.6 MB device -> host)
   e2e               clip_upload + clip_encode + clip_download (bench.py's `e2e`)
 
-Wall clock around issue + synchronize, warm; frames/s.  CEDAR_B200_UPLOAD_AHEAD is read by the library at open().
+Wall clock around issue + synchronize, warm; frames/s.
 """
 import json
 import os
@@ -67,7 +67,7 @@ def main():
         "encode+download": lambda e: (e.clip_encode(n, 0), e.clip_download(n)),
         "e2e": lambda e: (e.clip_upload(n), e.clip_encode(n, 0), e.clip_download(n)),
     }
-    res = {"upload_ahead": os.environ.get("CEDAR_B200_UPLOAD_AHEAD", "default"), "steps": steps, "handles": nh}
+    res = {"steps": steps, "handles": nh}
     for name, body in bodies.items():
         if only and name not in only:
             continue
