@@ -723,6 +723,31 @@ __device__ __forceinline__ void store_levels(int16_t *dst, const int16_t *lev)
     ((uint4 *)dst)[1] = b;
 }
 
+// Zig-zag scan index of raster position r of a 4x4 block: the inverse of h264_zigzag4x4.
+__device__ __forceinline__ int inv_zigzag4x4(int r)
+{
+    const uint8_t izz[16] = {0, 1, 5, 6, 2, 4, 7, 12, 3, 8, 11, 13, 9, 10, 14, 15};
+    return izz[r];
+}
+
+// Syntax records of chroma lanes 16..23 and lane 25, the same for inter and intra macroblocks: a chroma lane stores its
+// block's AC levels, nnz and DC level, and the first lane of each plane the nnz of the plane's DC block; lane 25 clears
+// the unused half of the chroma DC record.
+__device__ __forceinline__ void store_chroma_syntax(int16_t *cf, uint8_t *nn, int lane, const int16_t *lev, int nz,
+                                                    const ChromaOut &co)
+{
+    if (lane < 24) {
+        const int c = (lane - 16) >> 2, cb = lane & 3;
+        store_levels(cf + (18 + c * 4 + cb) * 16, lev);
+        nn[NNZ_CB + c * 4 + cb] = (uint8_t)nz;
+        cf[17 * 16 + c * 4 + cb] = (int16_t)co.zdc;
+        if (cb == 0)
+            nn[NNZ_CBDC + c] = (uint8_t)__popc(co.m_dc & (0xfu << (16 + 4 * c)));
+    } else if (lane == 25) {
+        *(uint4 *)(cf + 17 * 16 + 8) = make_uint4(0, 0, 0, 0);
+    }
+}
+
 // Quantiser constants of one lane's 4x4 block of an inter macroblock (luma lanes: QP, chroma lanes: QPc), so that luma
 // and chroma lanes run the transform / quantisation / reconstruction as one instruction stream.  Same arithmetic as
 // quant_block / dequant_ac (h264_core.cuh).
@@ -897,19 +922,11 @@ __global__ void __launch_bounds__(128) inter_kernel(Geom g, Step s, const uint8_
     if (luma) {
         store_levels(cf + lane * 16, lev);
         nn[lane] = (uint8_t)nz;
-    } else if (chroma) {
-        int c = (lane - 16) >> 2, cb = lane & 3;
-        store_levels(cf + (18 + c * 4 + cb) * 16, lev);
-        nn[NNZ_CB + c * 4 + cb] = (uint8_t)nz;
-        cf[17 * 16 + c * 4 + cb] = (int16_t)co.zdc;
-        if (cb == 0)
-            nn[NNZ_CBDC + c] = (uint8_t)__popc(co.m_dc & (0xfu << (16 + 4 * c)));
     } else if (lane == 24) {
         store_levels(cf + 16 * 16, lev); // zeros: no Intra16x16 DC block
         nn[NNZ_DC16] = 0;
-    } else if (lane == 25) {
-        *(uint4 *)(cf + 17 * 16 + 8) = make_uint4(0, 0, 0, 0);
-    }
+    } else
+        store_chroma_syntax(cf, nn, lane, lev, nz, co);
     if (lane == 0) {
         MbInfo m = me;
         m.type = MB_P16x16;
@@ -1030,7 +1047,6 @@ __device__ __forceinline__ bool intra4x4_trial(const Geom &g, I4Work &w, int lan
                                                bool has_leftmb, bool has_trmb, int top_kind, const uint8_t *top_modes,
                                                uint32_t cost16, int16_t *cf, int &cbp_out)
 {
-    const uint8_t izz[16] = {0, 1, 5, 6, 2, 4, 7, 12, 3, 8, 11, 13, 9, 10, 14, 15};
     const int r = lane & 15, x = r & 3, y = r >> 2, half = lane & 16, qp = g.qp;
     const int qbits = 15 + qp / 6, f = (1 << qbits) / 3, cls = pos_class(r);
     uint32_t cost4 = 0;
@@ -1105,7 +1121,7 @@ __device__ __forceinline__ bool intra4x4_trial(const Geom &g, I4Work &w, int lan
         const int z = quant1(v, h264_quant_mf[qp % 6][cls], f, qbits);
         const int n = __popc(__ballot_sync(0xffffffffu, z != 0) & 0xffffu);
         if (lane < 16)
-            cf[b * 16 + izz[r]] = (int16_t)z;
+            cf[b * 16 + inv_zigzag4x4(r)] = (int16_t)z;
         v = n ? dequant_ac(z, qp, cls) : 0;
         {
             const int rb = lane & ~3; // inverse transform, rows
@@ -1168,7 +1184,20 @@ __global__ void __launch_bounds__(INTRA_ROWS * 32) intra_kernel(Geom g, Step s, 
     const int bx = luma ? blk_x(lane) * 4 : (cb & 1) * 4, by = luma ? blk_y(lane) * 4 : (cb >> 1) * 4;
     const size_t plane_off = luma ? fo : fo + (size_t)g.W * g.H + (size_t)(chroma ? c : 0) * g.CW * g.CH;
     const int stride = luma ? g.W : g.CW, mbsz = luma ? 16 : 8;
-    const uint8_t izz[16] = {0, 1, 5, 6, 2, 4, 7, 12, 3, 8, 11, 13, 9, 10, 14, 15};
+
+    // Row `row` has finished macroblocks [0, n).  The CTA's last row releases its global flag, which the first row of the
+    // next CTA reads; the other rows fence their pixels (global stores, read back through L2 by the row below) before
+    // raising the shared counter.
+    auto publish = [&](int n) {
+        if (lane == 0) {
+            if (wrp == INTRA_ROWS - 1 || row == g.mbh - 1)
+                st_release(fl + row, n);
+            else {
+                __threadfence();
+                progress[wrp] = n;
+            }
+        }
+    };
 
     const bool try_i4 = g.intra4x4 && !pwant;
     for (int mbx = 0; mbx < g.mbw; mbx++) {
@@ -1176,14 +1205,7 @@ __global__ void __launch_bounds__(INTRA_ROWS * 32) intra_kernel(Geom g, Step s, 
         const size_t rec = (size_t)blockIdx.y * g.nmb + (size_t)row * g.mbw + mbx;
         if (pwant) {
             if (!pwant[rec]) { // stays inter: nothing to do but to let the row below pass
-                if (lane == 0) {
-                    if (wrp == INTRA_ROWS - 1 || row == g.mbh - 1)
-                        st_release(fl + row, mbx + 1);
-                    else {
-                        __threadfence();
-                        progress[wrp] = mbx + 1;
-                    }
-                }
+                publish(mbx + 1);
                 continue;
             }
             if (has_left) { // the left neighbour may be an inter macroblock: its column comes from the picture, not from this warp
@@ -1371,26 +1393,19 @@ __global__ void __launch_bounds__(INTRA_ROWS * 32) intra_kernel(Geom g, Step s, 
         uint8_t *nn = nnz + rec * NNZ_STRIDE;
         if (luma && use_i4) { // the levels were stored by the trial
             nn[lane] = i4w.nnzb[lane];
-            cf[16 * 16 + izz[lane]] = 0;
+            cf[16 * 16 + inv_zigzag4x4(lane)] = 0;
             i4[rec * 16 + lane] = i4w.mode[lane];
             i4w.left_mode[lane] = i4w.mode[lane];
         } else if (luma) {
             store_levels(cf + lane * 16, lev);
             nn[lane] = (uint8_t)(any_ac ? nz : 0);
-            cf[16 * 16 + izz[lane]] = (int16_t)zdc16;
+            cf[16 * 16 + inv_zigzag4x4(lane)] = (int16_t)zdc16;
             if (g.intra4x4)
                 i4[rec * 16 + lane] = 0;
-        } else if (chroma) {
-            store_levels(cf + (18 + c * 4 + cb) * 16, lev);
-            nn[NNZ_CB + c * 4 + cb] = (uint8_t)nz;
-            cf[17 * 16 + c * 4 + cb] = (int16_t)co.zdc;
-            if (cb == 0)
-                nn[NNZ_CBDC + c] = (uint8_t)__popc(co.m_dc & (0xfu << (16 + 4 * c)));
         } else if (lane == 24) {
             nn[NNZ_DC16] = (uint8_t)__popc(m_dc16 & 0xffffu);
-        } else if (lane == 25) {
-            *(uint4 *)(cf + 17 * 16 + 8) = make_uint4(0, 0, 0, 0);
-        }
+        } else
+            store_chroma_syntax(cf, nn, lane, lev, nz, co);
         int cmode = __shfl_sync(0xffffffffu, mode, 16);
         if (lane == 0) {
             MbInfo m;
@@ -1404,14 +1419,7 @@ __global__ void __launch_bounds__(INTRA_ROWS * 32) intra_kernel(Geom g, Step s, 
             mbi[rec] = m;
         }
         __syncwarp();
-        if (lane == 0) {
-            if (wrp == INTRA_ROWS - 1 || row == g.mbh - 1)
-                st_release(fl + row, mbx + 1); // read by the first row of the next CTA
-            else {
-                __threadfence(); // the pixels (global stores, read back through L2 by the row below) before the counter
-                progress[wrp] = mbx + 1;
-            }
-        }
+        publish(mbx + 1);
     }
 }
 
@@ -1527,15 +1535,6 @@ __device__ __forceinline__ void deblock_publisher(DeblockMail *mail, int *fl_min
     }
 }
 
-__device__ __forceinline__ void mail_wait(volatile int *p, int want, int lane)
-{
-    if (lane == 0)
-        while (*p < want)
-            __nanosleep(32);
-    __syncwarp();
-    __threadfence_block();
-}
-
 // One CTA filters `cta_rows` (<= DB_ROWS, chosen by the host so that the CTAs of a picture are equally tall: 68 rows = 4 x 17)
 // consecutive macroblock rows of one plane type (blockIdx.z: 0 luma, 1 Cb+Cr) of one
 // frame: warp j owns row j and hands the bottom rows of every finished macroblock to warp j+1 through a
@@ -1552,14 +1551,72 @@ struct DeblockRow {
     volatile int consumed;   // this row has consumed the top neighbours of macroblocks [0, consumed)
 };
 
-__device__ __forceinline__ void spin_until_ge(volatile int *p, int want, int lane)
+// Warp-collective wait for a shared-memory counter that another warp of the CTA raises: lane 0 polls until *p >= want,
+// sleeping `sleep_ns` between reads; the fence orders the warp's later reads after what the writer stored before.
+__device__ __forceinline__ void spin_until_ge(volatile int *p, int want, int lane, unsigned sleep_ns)
 {
     if (lane == 0)
         while (*p < want)
-            __nanosleep(20);
+            __nanosleep(sleep_ns);
     __syncwarp();
     __threadfence_block();
 }
+
+// The wavefront protocol of filtering warp j, the same for both plane types: where the top neighbours of a macroblock
+// come from, when its line-buffer slot may be overwritten, and the flags that report it stored.  Every member is called
+// by the whole warp.
+struct DeblockWave {
+    DeblockRow *rows;
+    DeblockMail *mail;
+    uint4 (*ring)[4];
+    int j, lane;
+    bool has_top, top_local, below_local, publish;
+
+    // Top neighbours of macroblock mbx from the row above's line buffer or the loader's ring; nullptr when there are
+    // none, or when the line buffer's are not needed because no horizontal edge is filtered.  The ring of the CTA's
+    // first row is consumed in order, so that row always waits.
+    __device__ __forceinline__ uint8_t *top(int mbx, bool any_h) const
+    {
+        uint8_t *t = nullptr;
+        if (top_local) {
+            if (any_h) {
+                spin_until_ge(&rows[j - 1].ready, mbx + 1, lane, 20);
+                t = (uint8_t *)rows[j - 1].lb[mbx % DB_NB];
+            } else
+                __syncwarp();
+        } else if (has_top) {
+            spin_until_ge(&mail->top_ready, mbx + 1, lane, 32);
+            t = (uint8_t *)ring[mbx & 1];
+        } else
+            __syncwarp();
+        return t;
+    }
+    // The line-buffer slot of mbx is free once the row below has consumed macroblock mbx - DB_NB.
+    __device__ __forceinline__ void wait_slot(int mbx) const
+    {
+        if (below_local)
+            spin_until_ge(&rows[j + 1].consumed, mbx - DB_NB + 1, lane, 20);
+        else
+            __syncwarp();
+    }
+    // Macroblock mbx is stored to the frame and, for the row below, to the line buffer.
+    __device__ __forceinline__ void done(int mbx) const
+    {
+        // the stores to the frame precede the flag: the row below stores this macroblock's bottom rows again after its
+        // top edge has filtered them, and that store has to land after this one
+        __threadfence_block();
+        __syncwarp();
+        if (lane == 0) {
+            rows[j].consumed = mbx + 1;
+            if (below_local)
+                rows[j].ready = mbx + 1; // macroblock mbx is final: nothing in this row touches it again
+            if (!top_local && has_top)
+                mail->top_consumed = mbx + 1;
+            if (publish)
+                mail->done = mbx + 1;
+        }
+    }
+};
 
 __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Step s, const uint8_t *__restrict__ unf,
                                                                       uint8_t *rec, const uint8_t *__restrict__ bs,
@@ -1612,7 +1669,8 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
 
     const int j = warp, row = row0 + j;
     DeblockRow &me = rows[j];
-    const bool has_top = row > 0, top_local = j > 0, below_local = j + 1 < nr, publish = j == nr - 1 && row + 1 < g.mbh;
+    const bool has_top = row > 0, below_local = j + 1 < nr;
+    const DeblockWave wave = {rows, &mail, ring, j, lane, has_top, j > 0, below_local, j == nr - 1 && row + 1 < g.mbh};
     const uint4 *fbs = (const uint4 *)bs + ((size_t)blockIdx.y * g.nmb + (size_t)row * g.mbw) * 2;
 
     if (!chroma) {
@@ -1671,19 +1729,7 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
                 t[1] = w[1], t[2] = w[2], t[3] = w[3], t[4] = w[4];
             }
             DB_MARK(1);
-            // ---- top neighbours (the ring of the CTA's first row is consumed in order, so that row always waits) ----
-            uint8_t *top = nullptr;
-            if (top_local) {
-                if (any_h) {
-                    spin_until_ge(&rows[j - 1].ready, mbx + 1, lane);
-                    top = (uint8_t *)rows[j - 1].lb[mbx % DB_NB];
-                } else
-                    __syncwarp();
-            } else if (has_top) {
-                mail_wait(&mail.top_ready, mbx + 1, lane);
-                top = (uint8_t *)ring[mbx & 1];
-            } else
-                __syncwarp();
+            uint8_t *top = wave.top(mbx, any_h);
             DB_MARK(2);
             // ---- horizontal edges, lane = column: the 20-sample column stays in registers ----
             if (lane < 16 && any_h) {
@@ -1731,10 +1777,7 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
                 }
             }
             DB_MARK(3);
-            if (below_local) // the slot is free once the row below has consumed macroblock mbx - DB_NB
-                spin_until_ge(&rows[j + 1].consumed, mbx - DB_NB + 1, lane);
-            else
-                __syncwarp();
+            wave.wait_slot(mbx);
             DB_MARK(4);
             if (lane < 16) {
                 const uint32_t *t = me.tile + lane * 6;
@@ -1747,19 +1790,7 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
                 int r = lane - 15; // top rows 1..3 were modified
                 *(uint4 *)(rec + fo + (size_t)(y0 - 4 + r) * g.W + x0) = ((const uint4 *)top)[r];
             }
-            // the stores to the frame precede the flag: the row below stores this macroblock's rows 13..15 again after its
-            // top edge has filtered them, and that store has to land after this one
-            __threadfence_block();
-            __syncwarp();
-            if (lane == 0) {
-                me.consumed = mbx + 1;
-                if (below_local)
-                    me.ready = mbx + 1; // macroblock mbx is final: nothing in this row touches it again
-                if (!top_local && has_top)
-                    mail.top_consumed = mbx + 1;
-                if (publish)
-                    mail.done = mbx + 1;
-            }
+            wave.done(mbx);
             DB_MARK(5);
         }
 #ifdef DB_PROFILE
@@ -1807,18 +1838,7 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
                 }
                 t[1] = w1, t[2] = w2;
             }
-            uint8_t *topb = nullptr; // [plane][2 rows][8 bytes]
-            if (top_local) {
-                if (any_h) {
-                    spin_until_ge(&rows[j - 1].ready, mbx + 1, lane);
-                    topb = (uint8_t *)rows[j - 1].lb[mbx % DB_NB];
-                } else
-                    __syncwarp();
-            } else if (has_top) {
-                mail_wait(&mail.top_ready, mbx + 1, lane);
-                topb = (uint8_t *)ring[mbx & 1];
-            } else
-                __syncwarp();
+            uint8_t *topb = wave.top(mbx, any_h); // [plane][2 rows][8 bytes]
             uint8_t *top = topb + pl * 16;
             if (lane < 16 && any_h) { // horizontal edges at chroma y = 0, 4: lane = (plane, column)
                 uint8_t *col = tb + 4 + r8;
@@ -1856,10 +1876,7 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
                     }
                 }
             }
-            if (below_local)
-                spin_until_ge(&rows[j + 1].consumed, mbx - DB_NB + 1, lane);
-            else
-                __syncwarp();
+            wave.wait_slot(mbx);
             if (lane < 16) {
                 uint8_t *o = rec + po + (size_t)(y0 + r8) * g.CW + x0;
                 const uint2 mine = make_uint2(tw[r8 * 3 + 1], tw[r8 * 3 + 2]);
@@ -1871,17 +1888,7 @@ __global__ void __launch_bounds__((DB_ROWS + 2) * 32) deblock_kernel(Geom g, Ste
                 *(uint2 *)(rec + fo + (size_t)g.W * g.H + (size_t)p2 * g.CW * g.CH + (size_t)(y0 - 1) * g.CW + x0) =
                     ((const uint2 *)topb)[p2 * 2 + 1];
             }
-            __threadfence_block();
-            __syncwarp();
-            if (lane == 0) {
-                me.consumed = mbx + 1;
-                if (below_local)
-                    me.ready = mbx + 1;
-                if (!top_local && has_top)
-                    mail.top_consumed = mbx + 1;
-                if (publish)
-                    mail.done = mbx + 1;
-            }
+            wave.done(mbx);
         }
     }
 }
@@ -1980,27 +1987,24 @@ __global__ void entropy_size_kernel(Geom g, Step s, int frame_i, const MbInfo *_
     eb.mb_size[(size_t)blockIdx.y * (nitems + 1) + i] = n;
 }
 
-// Exclusive prefix sum of the item sizes of a picture (one 1024-thread CTA per lane) + per-slice totals.
-__global__ void __launch_bounds__(1024) entropy_scan_kernel(Geom g, Step s, EntropyBufs eb)
+// Exclusive scan of in[0, n) into out[0, n) by one 1024-thread CTA, starting at `carry`, in chunks of 1024: a warp scan,
+// a scan of the warp sums, then the carry into the next chunk.  Each thread reads its element before it writes it, so
+// in == out is allowed.  Returns carry + the sum of in[0, n) to every thread.
+template <class In, class Acc>
+__device__ __forceinline__ Acc block_exclusive_scan(const In *in, Acc *out, unsigned n, Acc carry)
 {
-    int f = lane_frame(s, blockIdx.y);
-    if (f < 0)
-        return;
-    __shared__ uint32_t warp_sum[32];
-    __shared__ uint32_t carry_s;
-    __shared__ unsigned long long pool_off;
-    const int n = g.nmb + g.nslices, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t *in = eb.mb_size + (size_t)blockIdx.y * (n + 1);
-    uint32_t *out = eb.mb_off + (size_t)blockIdx.y * (n + 1);
+    __shared__ Acc warp_sum[32];
+    __shared__ Acc carry_s;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0)
-        carry_s = 0;
+        carry_s = carry;
     __syncthreads();
-    for (int start = 0; start < n; start += 1024) {
-        int i = start + tid;
-        uint32_t v = i < n ? in[i] : 0, x = v;
+    for (unsigned start = 0; start < n; start += 1024) {
+        const unsigned i = start + tid;
+        Acc v = i < n ? (Acc)in[i] : 0, x = v;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-            uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
+            Acc y = __shfl_up_sync(0xffffffffu, x, o);
             if (lane >= o)
                 x += y;
         }
@@ -2008,18 +2012,17 @@ __global__ void __launch_bounds__(1024) entropy_scan_kernel(Geom g, Step s, Entr
             warp_sum[warp] = x;
         __syncthreads();
         if (warp == 0) {
-            uint32_t ws = warp_sum[lane], z = ws;
+            Acc ws = warp_sum[lane], z = ws;
 #pragma unroll
             for (int o = 1; o < 32; o <<= 1) {
-                uint32_t y = __shfl_up_sync(0xffffffffu, z, o);
+                Acc y = __shfl_up_sync(0xffffffffu, z, o);
                 if (lane >= o)
                     z += y;
             }
             warp_sum[lane] = z - ws; // exclusive
         }
         __syncthreads();
-        uint32_t carry = carry_s;
-        uint32_t incl = carry + warp_sum[warp] + x;
+        Acc incl = carry_s + warp_sum[warp] + x;
         if (i < n)
             out[i] = incl - v;
         __syncthreads();
@@ -2027,8 +2030,20 @@ __global__ void __launch_bounds__(1024) entropy_scan_kernel(Geom g, Step s, Entr
             carry_s = incl;
         __syncthreads();
     }
+    return carry_s;
+}
+
+// Exclusive prefix sum of the item sizes of a picture (one 1024-thread CTA per lane) + per-slice totals.
+__global__ void __launch_bounds__(1024) entropy_scan_kernel(Geom g, Step s, EntropyBufs eb)
+{
+    int f = lane_frame(s, blockIdx.y);
+    if (f < 0)
+        return;
+    __shared__ unsigned long long pool_off;
+    const int n = g.nmb + g.nslices, tid = threadIdx.x;
+    uint32_t *out = eb.mb_off + (size_t)blockIdx.y * (n + 1);
+    const uint32_t total = block_exclusive_scan(eb.mb_size + (size_t)blockIdx.y * (n + 1), out, n, 0u);
     if (tid == 0) {
-        const uint32_t total = carry_s;
         out[n] = total;
         if (g.cabac) { // one pool allocation per picture; its slices lie back to back
             unsigned long long off = atomicAdd(eb.bins_cursor, (unsigned long long)((total + 7u) & ~7u));
@@ -2753,107 +2768,33 @@ __global__ void __launch_bounds__(1024) epb_scan_kernel(int nframes, const uint3
                                                         uint32_t *__restrict__ nal_bytes, ParamSets ps, int nslices,
                                                         int gop_len, int first_frame_index)
 {
-    int f = blockIdx.x;
-    __shared__ uint32_t warp_sum[32];
-    __shared__ uint32_t carry_s;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    unsigned n = (rbsp_len[f] + EPB_CHUNK - 1) / EPB_CHUNK;
+    const int f = blockIdx.x;
     uint32_t *c = chunk_cnt + (size_t)f * chunks_per_frame;
-    if (tid == 0)
-        carry_s = 0;
-    __syncthreads();
-    for (unsigned start = 0; start < n; start += 1024) {
-        unsigned i = start + tid;
-        uint32_t v = i < n ? c[i] : 0, x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o)
-                x += y;
-        }
-        if (lane == 31)
-            warp_sum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            uint32_t ws = warp_sum[lane], z = ws;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                uint32_t y = __shfl_up_sync(0xffffffffu, z, o);
-                if (lane >= o)
-                    z += y;
-            }
-            warp_sum[lane] = z - ws;
-        }
-        __syncthreads();
-        uint32_t incl = carry_s + warp_sum[warp] + x;
-        if (i < n)
-            c[i] = incl - v;
-        __syncthreads();
-        if (tid == 1023)
-            carry_s = incl;
-        __syncthreads();
-    }
-    if (tid == 0)
-        nal_bytes[f] = rbsp_len[f] ? 5 + rbsp_len[f] + carry_s + // start code + NAL header + payload (+ SPS, PPS in front)
+    const uint32_t epb = block_exclusive_scan(c, c, (rbsp_len[f] + EPB_CHUNK - 1) / EPB_CHUNK, 0u);
+    if (threadIdx.x == 0)
+        nal_bytes[f] = rbsp_len[f] ? 5 + rbsp_len[f] + epb + // start code + NAL header + payload (+ SPS, PPS in front)
                                          (has_param_sets(ps, f, nslices, gop_len, first_frame_index) ? ps.len : 0)
                                    : 0;
 }
 
-// Single CTA: exclusive scan of the per-frame NAL sizes -> offsets in the packed stream.
+// Single CTA: exclusive scan of the NAL sizes (one per slice NAL) -> offsets in the packed stream.
 // frame_bytes[f] additionally counts the parameter sets that precede frame 0 (cedar.c:1058-1061).
 __global__ void __launch_bounds__(1024) pack_scan_kernel(int nunits, int nslices, const uint32_t *__restrict__ nal_bytes,
                                                          unsigned prefix_bytes, unsigned long long *nal_off,
                                                          int *__restrict__ frame_bytes, unsigned long long *total,
                                                          unsigned long long out_cap, int *error)
 {
-    const int nframes = nunits; // scanned entries: one per slice NAL
-    __shared__ unsigned long long warp_sum[32];
-    __shared__ unsigned long long carry_s;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0)
-        carry_s = prefix_bytes;
-    __syncthreads();
-    for (int start = 0; start < nframes; start += 1024) {
-        int i = start + tid;
-        unsigned long long v = i < nframes ? nal_bytes[i] : 0, x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o)
-                x += y;
-        }
-        if (lane == 31)
-            warp_sum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            unsigned long long ws = warp_sum[lane], z = ws;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                unsigned long long y = __shfl_up_sync(0xffffffffu, z, o);
-                if (lane >= o)
-                    z += y;
-            }
-            warp_sum[lane] = z - ws;
-        }
-        __syncthreads();
-        unsigned long long incl = carry_s + warp_sum[warp] + x;
-        if (i < nframes)
-            nal_off[i] = incl - v;
-        __syncthreads();
-        if (tid == 1023)
-            carry_s = incl;
-        __syncthreads();
-    }
+    const int tid = threadIdx.x;
+    const unsigned long long end_all = block_exclusive_scan(nal_bytes, nal_off, nunits, (unsigned long long)prefix_bytes);
     // bytes per picture = its slice NALs (+ the parameter sets in front of picture 0)
-    const unsigned long long end_all = carry_s;
     for (int fr = tid; fr < nunits / nslices; fr += 1024) {
         unsigned long long b = fr == 0 ? 0 : nal_off[(size_t)fr * nslices];
         unsigned long long e = (fr + 1) * nslices < nunits ? nal_off[(size_t)(fr + 1) * nslices] : end_all;
         frame_bytes[fr] = (int)(e - b);
     }
     if (tid == 0) {
-        *total = carry_s;
-        if (carry_s > out_cap) {
+        *total = end_all;
+        if (end_all > out_cap) {
             atomicExch(error, 4);
             *total = 0;
         }

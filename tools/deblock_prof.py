@@ -1,5 +1,5 @@
 """Diagnosis: per-phase clock64 timing of the luma deblocking warp (needs tools/libcedar_prof.so built with
--DDEBLOCK_PROFILE)."""
+-DDB_PROFILE)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
