@@ -552,6 +552,9 @@ int encode_step(cedar_b200_handle *h, const Step &s, int t, int gop_pos0, int st
         if (h->count && h->no_prune) // the measurement without pruning: no bound either
             ms.bound = 0;
         ms.exec_count = h->count ? h->d_counters : nullptr;
+#ifdef ME_PROFILE
+        ms.exec_count = h->d_counters; // the phase cycles of the product kernel (kernels.cuh, ME_MARK)
+#endif
         const dim3 me_grid((g.mbw + ms.nstrip - 1) / ms.nstrip, (g.mbh + ms.nrow - 1) / ms.nrow, nl);
         const size_t me_smem = me_smem_bytes(g.R, ms.nstrip);
         const auto me = me_kernel_for(ms.RSW, h->count);

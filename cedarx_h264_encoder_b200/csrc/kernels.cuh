@@ -236,6 +236,7 @@ struct MeShape {
     int nstrip, lstrip, nrow, RSW, CWs, WR, nd, nfull, nleft, ndyg; // lstrip = log2(nstrip)
     int bound;                       // block-sum bound path (me_bound_path)
     int tpw, trows;                  // its table: words per phase row, rows
+    int tseg, tnseg;                 // its build: rows per segment, segments (one pass of the CTA's threads, me_shape)
     uint32_t nd_magic;               // __umulhi(i, nd_magic) == i / nd for the bound stage's item indices
     int noprune;                     // measurement only (CEDAR_B200_NO_PRUNE): every candidate is accumulated to the end
     // measurement only (profiling on), else null: [0] executed VABSDIFF4 lane-instructions, [1] candidates bounded,
@@ -256,6 +257,11 @@ inline MeShape me_shape(int R)
     m.bound = me_bound_path(R);
     m.tpw = me_tab_pw(R, m.nstrip);
     m.trows = me_tab_rows(R);
+    // the table build's thread = (segment, phase, word): the shortest segments that still give every thread at most one
+    // item (R = 16: 11 segments of 9 rows x 28 words = 308 items), so the CTA builds the table in one pass
+    const int tw = 4 * m.tpw, per_col = ME_THREADS / tw > 0 ? ME_THREADS / tw : 1;
+    m.tseg = (m.trows + per_col - 1) / per_col;
+    m.tnseg = (m.trows + m.tseg - 1) / m.tseg;
     m.nd_magic = (uint32_t)(((1ull << 32) + (unsigned)m.nd - 1) / (unsigned)m.nd); // exact for i < 2^32 / nd
     m.noprune = 0;
     m.exec_count = nullptr;
@@ -292,36 +298,59 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
     const uint8_t *srcY = src + (size_t)blockIdx.z * g.frame_bytes;
     const uint8_t *refY = ref + (size_t)blockIdx.z * g.frame_bytes;
     uint32_t *cur_s = sm, *cp = sm + 64 * nmb, *item_tab = cp + 4 * CWs;
-    const int tid = threadIdx.x;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nwarps = ME_THREADS / 32;
+#ifdef ME_PROFILE
+    // Measurement build (-DME_PROFILE): clock64 marks at the phase boundaries, behind a barrier so that a phase ends when
+    // its slowest warp does; thread 0 adds them to exec_count[480 + phase] and counts the tile in exec_count[487]
+    unsigned long long prof_pt[7] = {0, 0, 0, 0, 0, 0, 0};
+    long long prof_t = clock64();
+#define ME_MARK(i)                                                                                                     \
+    {                                                                                                                  \
+        __syncthreads();                                                                                               \
+        const long long now_ = clock64();                                                                              \
+        prof_pt[i] += (unsigned long long)(now_ - prof_t);                                                             \
+        prof_t = now_;                                                                                                 \
+    }
+#else
+#define ME_MARK(i)
+#endif
 
     // Tables that take every division and every bit-length computation out of the task loop; they only depend on the
     // configuration, so the host builds them once (me_build_tables) and every CTA copies them; tasks of macroblocks
-    // beyond the picture edge are skipped (vmask).
+    // beyond the picture edge are skipped (vmask).  The task tables are read by the exhaustive search only: a tile on
+    // the bound path copies them when its list overflows.
     const int nleft = ms.nleft, ndyg = ms.ndyg;
     const int ntask_full = ms.nfull * ndyg;               // per macroblock: 32 columns x one row group
     const int nitems_left = nleft * ndyg * nmb;        // left-over columns of all macroblocks, one item per lane
-    for (int i = tid; i < 136; i += ME_THREADS)
-        mvcost[i] = tabs[i];
-    for (int i = tid; i < ntask_full * nmb; i += ME_THREADS)
-        task_tab[i] = tabs[136 + i];
-    for (int i = tid; i < ((nitems_left + 31) & ~31); i += ME_THREADS)
-        item_tab[i] = i < nitems_left ? tabs[136 + ME_TASK_WORDS + i] : 0xffffffffu;
-    if (tid < ME_MAX_MB)
-        mb_best[tid] = 0xffffffffu;
-    for (int i = tid; i < 64 * nmb; i += ME_THREADS) { // current blocks: [mb][row][4 words]
-        int m = i >> 6, row = (i >> 2) & 15, k = i & 3;
-        if ((vmask >> m) & 1)
-            cur_s[i] = *(const uint32_t *)(srcY + (size_t)(y0 + 16 * (m >> ls) + row) * g.W + x0 + 16 * (m & (nstrip - 1)) + 4 * k);
-    }
+    auto copy_task_tables = [&]() {
+        for (int i = tid; i < ntask_full * nmb; i += ME_THREADS)
+            task_tab[i] = tabs[136 + i];
+        for (int i = tid; i < ((nitems_left + 31) & ~31); i += ME_THREADS)
+            item_tab[i] = i < nitems_left ? tabs[136 + ME_TASK_WORDS + i] : 0xffffffffu;
+    };
     const bool bound = kRSW != 43 && ms.bound; // kRSW = 43 is R > 32, never on the bound path
-    if (tid == 0)
-        list_n = 0;
+
     // Window staging: warp = window row (round robin), lane = 32-bit word of the row.  Each lane fetches its
     // word and the next one (the second fetch hits L1) and builds the three byte-shifted copies in
     // registers; no integer division, no shared-memory round trip.  plain: copy 0, shifted: copies 1..3.
-    auto stage = [&](const bool plain, const bool shifted) {
-        const int warp_ = tid >> 5, lane_ = tid & 31;
-        const bool interior_x = x0 - R >= 0 && x0 - R + 4 * RSW + 4 <= g.W && !((x0 - R) & 3);
+    // Interior tiles whose window starts on a 16-byte boundary (R = 16: all of them), is at most 32 words wide and at
+    // most three passes tall: eight lanes per row, four rows per warp pass, one 16-byte load per lane -- a third of the
+    // instructions of the word-per-lane loop.  The four rows of a pass land in different banks (RSW is odd).  The
+    // loads of all passes are issued before the first store (vec_load), so a lane waits for one round trip, not three.
+    const bool interior_x = x0 - R >= 0 && x0 - R + 4 * RSW + 4 <= g.W && !((x0 - R) & 3);
+    const int nq = (RSW + 4) >> 2; // 16-byte groups that hold window words 0 .. RSW
+    constexpr int kPasses = 3;
+    const bool vec = interior_x && !((x0 - R) & 15) && RSW < 32 && x0 - R + 16 * nq <= g.W && WR <= 4 * nwarps * kPasses;
+    auto vec_load = [&](uint4 *v) {
+#pragma unroll
+        for (int p = 0; p < kPasses; p++) {
+            const int r = 4 * (warp + nwarps * p) + (lane >> 3), q = lane & 7;
+            v[p] = make_uint4(0, 0, 0, 0);
+            if (vec && r < WR && q < nq)
+                v[p] = *(const uint4 *)(refY + (size_t)clip3_(0, g.H - 1, y0 - R + r) * g.W + (x0 - R) + 16 * q);
+        }
+    };
+    auto stage = [&](const uint4 *v, const bool plain, const bool shifted) {
         auto fetch = [&](const uint8_t *row, int k) -> uint32_t { // window word k of a row, edge clamped
             const int fx = x0 - R + 4 * k;
             if (interior_x)
@@ -332,20 +361,13 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
                 v |= (uint32_t)row[clip3_(0, g.W - 1, fx + i)] << (8 * i);
             return v;
         };
-        // Interior tiles whose window starts on a 16-byte boundary (R = 16: all of them) and is at most 32 words wide:
-        // eight lanes per row, four rows per warp pass, one 16-byte load per lane -- a third of the instructions of the
-        // word-per-lane loop below.  The four rows of a pass land in different banks (RSW is odd).
-        const int nq = (RSW + 4) >> 2; // 16-byte groups that hold window words 0 .. RSW
-        const bool vec = interior_x && !((x0 - R) & 15) && RSW < 32 && x0 - R + 16 * nq <= g.W;
         if (vec) {
-            const int sub = lane_ >> 3, q = lane_ & 7;
-            for (int r4 = 4 * warp_; r4 < WR; r4 += 4 * (ME_THREADS / 32)) {
-                const int r = r4 + sub;
+            const int sub = lane >> 3, q = lane & 7;
+#pragma unroll
+            for (int p = 0; p < kPasses; p++) {
+                const int r = 4 * (warp + nwarps * p) + sub;
                 const bool on = r < WR && q < nq;
-                uint4 v = make_uint4(0, 0, 0, 0);
-                if (on)
-                    v = *(const uint4 *)(refY + (size_t)clip3_(0, g.H - 1, y0 - R + r) * g.W + (x0 - R) + 16 * q);
-                const uint32_t w[5] = {v.x, v.y, v.z, v.w, __shfl_down_sync(0xffffffffu, v.x, 1)};
+                const uint32_t w[5] = {v[p].x, v[p].y, v[p].z, v[p].w, __shfl_down_sync(0xffffffffu, v[p].x, 1)};
                 uint32_t *d = cp + r * RSW + 4 * q;
 #pragma unroll
                 for (int i = 0; i < 4; i++)
@@ -360,13 +382,13 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
                     }
             }
         }
-        for (int r = vec ? WR : warp_; r < WR; r += ME_THREADS / 32) {
+        for (int r = vec ? WR : warp; r < WR; r += ME_THREADS / 32) {
             const uint8_t *row = refY + (size_t)clip3_(0, g.H - 1, y0 - R + r) * g.W;
             for (int k0 = 0; k0 < RSW; k0 += 32) {
-                const int k = k0 + lane_;
+                const int k = k0 + lane;
                 const uint32_t lo = k <= RSW ? fetch(row, k) : 0u;
                 uint32_t hi = __shfl_down_sync(0xffffffffu, lo, 1); // the next word is the neighbouring lane's
-                if (lane_ == 31 && k < RSW)
+                if (lane == 31 && k < RSW)
                     hi = fetch(row, k + 1);
                 if (k < RSW) {
                     uint32_t *d = cp + r * RSW + k;
@@ -381,13 +403,45 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
             }
         }
     };
-    stage(true, !bound);
+    // One round of global loads per thread, all issued before its first shared store: a word of the vector-cost table,
+    // a 16-byte row of a current block ([mb][row][4 words]: thread = mb * 16 + row), the window rows of its warp and the
+    // motion vectors of the seeds' co-located macroblocks (one warp pass per macroblock, at most two per warp).
+    static_assert(ME_MAX_MB * 16 <= ME_THREADS && ME_MAX_MB <= 2 * (ME_THREADS / 32), "me_kernel: one load round");
+    const uint32_t cost_w = tid < 136 ? tabs[tid] : 0u;
+    uint4 cur_w = make_uint4(0, 0, 0, 0);
+    const bool cur_on = tid < 16 * nmb && ((vmask >> (tid >> 4)) & 1);
+    if (cur_on) {
+        const int m = tid >> 4;
+        cur_w = *(const uint4 *)(srcY + (size_t)(y0 + 16 * (m >> ls) + (tid & 15)) * g.W + x0 + 16 * (m & (nstrip - 1)));
+    }
+    uint4 wv[kPasses];
+    vec_load(wv);
+    int seed_mv[2] = {0, 0}; // mv[0] | mv[1] << 16 of MbInfo
+#pragma unroll
+    for (int k = 0; k < 2; k++) {
+        const int m = warp + nwarps * k;
+        if (lane >= 16 && m < nmb && ((vmask >> m) & 1))
+            seed_mv[k] = *(const int *)mbi_prev[(size_t)blockIdx.z * g.nmb + (size_t)(mby0 + (m >> ls)) * g.mbw + mbx0 +
+                                                 (m & (nstrip - 1))].mv;
+    }
+    if (tid < 136)
+        mvcost[tid] = cost_w;
+    if (cur_on)
+        ((uint4 *)cur_s)[tid] = cur_w;
+    if (tid < ME_MAX_MB)
+        mb_best[tid] = 0xffffffffu;
+    if (tid == 0)
+        list_n = 0;
+    if (!bound)
+        copy_task_tables();
+    ME_MARK(0);
+    stage(wv, true, !bound);
     __syncthreads();
+    ME_MARK(1);
     // copy 0 read at byte offset ox & 3 (what copy ox & 3 holds): the seeds and the bound path's SAD stage
     auto win = [&](const uint32_t *p, int sh) { return __funnelshift_r(p[0], p[1], sh); };
     unsigned nabs = 0; // measurement build: VABSDIFF4 lane-instructions of the bound path
 
-    const int warp = tid >> 5, lane = tid & 31, nwarps = ME_THREADS / 32;
     // Seed the running minimum with two real candidates per macroblock -- the zero vector and the vector the
     // co-located macroblock had in the previous frame (any value is fine: it only has to be a candidate of the
     // search) -- so that the bound stage can reject candidates outright and the SAD loops can drop a task as soon as the
@@ -395,15 +449,16 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
     // bound of the final key: the argmin, and with it the bitstream, is unchanged.
     // one warp pass per macroblock: lanes 0..15 take the rows of the zero-vector seed, lanes 16..31 those of the
     // co-located one
-    for (int m = warp; m < nmb; m += nwarps) {
+#pragma unroll
+    for (int k = 0; k < 2; k++) {
+        const int m = warp + nwarps * k;
         const int mc = m & (nstrip - 1), mr = m >> ls, half = lane >> 4, l16 = lane & 15;
-        if (!((vmask >> m) & 1))
+        if (m >= nmb || !((vmask >> m) & 1))
             continue;
         int ox = R, oy = R;
         if (half) {
-            const MbInfo pv = mbi_prev[(size_t)blockIdx.z * g.nmb + (size_t)(mby0 + mr) * g.mbw + mbx0 + mc];
-            ox = clip3_(0, nd - 1, (pv.mv[0] >> 2) + R);
-            oy = clip3_(0, nd - 1, (pv.mv[1] >> 2) + R);
+            ox = clip3_(0, nd - 1, ((int)(int16_t)seed_mv[k] >> 2) + R);
+            oy = clip3_(0, nd - 1, (seed_mv[k] >> 18) + R);
         }
         uint32_t a = 0;
         const uint32_t *wp = cp + (oy + 16 * mr + l16) * RSW + 4 * mc + (ox >> 2);
@@ -437,13 +492,12 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
         }
         for (int i = tid; i < 3 * tw; i += ME_THREADS)
             tab[ms.trows * tw + i] = 0;
-        // thread = (segment of kSeg table rows, phase c, word w): four running rows of 4-pixel sums per column, so every
-        // window word is read once per segment.  Bytes of positions no candidate reaches are 0.
-        constexpr int kSeg = 12;
-        const int xs_max = 16 * (nstrip - 1) + 2 * R + 12, nseg = (ms.trows + kSeg - 1) / kSeg;
-        for (int it = tid; it < nseg * tw; it += ME_THREADS) {
+        // thread = (segment of ms.tseg table rows, phase c, word w): four running rows of 4-pixel sums per column, so
+        // every window word is read once per segment.  Bytes of positions no candidate reaches are 0.
+        const int xs_max = 16 * (nstrip - 1) + 2 * R + 12;
+        for (int it = tid; it < ms.tnseg * tw; it += ME_THREADS) {
             const int seg = it / tw, col = it - seg * tw, c = col / tpw, w = col - c * tpw;
-            const int y0 = seg * kSeg, y1 = imin_(y0 + kSeg, ms.trows), sh = 8 * c;
+            const int y0 = seg * ms.tseg, y1 = imin_(y0 + ms.tseg, ms.trows), sh = 8 * c;
             int idx[4];
             uint32_t valid = 0;
 #pragma unroll
@@ -479,6 +533,7 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
         }
     }
     __syncthreads();
+    ME_MARK(2);
     bool fallback = !bound;
     unsigned nbounded = 0, nsad = 0; // measurement build
     if (bound) {
@@ -530,39 +585,44 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
         if (kCount)
             nabs += 4 * nbounded;
         __syncthreads();
+        ME_MARK(3);
         fallback = list_n > ME_LIST_CAP;
         if (!fallback) {
-            // SAD stage: one listed candidate per thread, read from copy 0, with a partial-cost exit after eight rows
-            const int n = list_n;
-            for (int i = tid; i < n; i += ME_THREADS) {
-                const uint32_t e = list[i];
+            // SAD stage: four lanes per listed candidate, eight candidates per warp pass, read from copy 0; lane l of a
+            // candidate takes block rows l, l + 4, l + 8, l + 12 (four window words each by funnel shift, a chain of 16
+            // VABSDIFF4), two shuffles sum them.  The key (cost << 15 | rank) does not depend on the order in which
+            // candidates reach the minimum.
+            const int n = list_n, sub = lane & 3;
+            for (int i0 = 8 * warp; i0 < n; i0 += 8 * nwarps) {
+                const int i = i0 + (lane >> 2);
+                const uint32_t e = list[i < n ? i : i0]; // lanes past the list repeat the pass's first candidate
                 const int m = (int)(e & 15), ox = (int)((e >> 4) & 255), oy = (int)(e >> 12), sh = 8 * (ox & 3);
-                const uint32_t *wp = cp + (oy + 16 * (m >> ls)) * RSW + 4 * (m & (nstrip - 1)) + (ox >> 2);
-                const uint4 *cu = (const uint4 *)(cur_s + 64 * m);
-                const uint32_t rank = (uint32_t)(oy * nd + ox);
-                uint32_t acc = mvcost[ox] + mvcost[oy];
-                bool dead = false;
+                const uint32_t *wp = cp + (oy + 16 * (m >> ls) + sub) * RSW + 4 * (m & (nstrip - 1)) + (ox >> 2);
+                const uint4 *cu = (const uint4 *)(cur_s + 64 * m) + sub;
+                uint32_t a = 0;
 #pragma unroll
-                for (int r = 0; r < 16; r++) {
-                    if (r == 8) {
-                        dead = ((acc << 15) | rank) > *(volatile uint32_t *)&mb_best[m];
-                        if (dead)
-                            break;
-                    }
-                    const uint4 cw = cu[r];
-                    const uint32_t *p = wp + r * RSW;
-                    acc = sad4_acc(win(p, sh), cw.x, acc);
-                    acc = sad4_acc(win(p + 1, sh), cw.y, acc);
-                    acc = sad4_acc(win(p + 2, sh), cw.z, acc);
-                    acc = sad4_acc(win(p + 3, sh), cw.w, acc);
+                for (int r = 0; r < 4; r++) {
+                    const uint4 cw = cu[4 * r];
+                    const uint32_t *p = wp + 4 * r * RSW;
+                    a = sad4_acc(win(p, sh), cw.x, a);
+                    a = sad4_acc(win(p + 1, sh), cw.y, a);
+                    a = sad4_acc(win(p + 2, sh), cw.z, a);
+                    a = sad4_acc(win(p + 3, sh), cw.w, a);
                 }
-                if (kCount)
-                    nabs += dead ? 32 : 64, nsad++;
-                if (!dead)
-                    atomicMin(&mb_best[m], (acc << 15) | rank);
+                a += __shfl_xor_sync(0xffffffffu, a, 1);
+                a += __shfl_xor_sync(0xffffffffu, a, 2);
+                if (sub == 0 && i < n) {
+                    atomicMin(&mb_best[m], ((a + mvcost[ox] + mvcost[oy]) << 15) | (uint32_t)(oy * nd + ox));
+                    if (kCount)
+                        nabs += 64, nsad++;
+                }
             }
+            ME_MARK(4);
         } else {
-            stage(false, true); // the exhaustive search below reads the byte-shifted copies
+            // the exhaustive search below reads the task tables and the byte-shifted copies
+            vec_load(wv);
+            copy_task_tables();
+            stage(wv, false, true);
             __syncthreads();
         }
     }
@@ -661,6 +721,7 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
             atomicMin(&mb_best[m], key);
     }
     __syncthreads();
+    ME_MARK(5);
     if (tid < nmb && ((vmask >> tid) & 1)) {
         const uint32_t b = mb_best[tid];
         int rank = (int)(b & 0x7fff);
@@ -673,6 +734,15 @@ __global__ void __launch_bounds__(ME_THREADS, kCount ? 1 : 4) me_kernel(Geom g, 
         mi.pad = b >> 15; // best cost, for statistics
         mbi[(size_t)blockIdx.z * g.nmb + (size_t)(mby0 + (tid >> ls)) * g.mbw + mbx0 + (tid & (nstrip - 1))] = mi;
     }
+#ifdef ME_PROFILE
+    ME_MARK(6);
+    if (tid == 0 && ms.exec_count) {
+        for (int i = 0; i < 7; i++)
+            atomicAdd(ms.exec_count + 480 + i, prof_pt[i]);
+        atomicAdd(ms.exec_count + 487, 1ull);
+    }
+#endif
+#undef ME_MARK
 }
 
 // ================================================================================================
